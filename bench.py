@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — MD steps/s of the non-bonded + VelocityVerlet hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3] [--dump-outputs DIR]
 
 A "step" is one VelocityVerlet MD step (kick, drift, neighbour policy, pairwise forces, kick, CM removal)
 of the workload; at N=1 the workload is BASELINE config[1]: the 256 000-atom argon LJ fluid, cubic PBC,
@@ -19,6 +19,10 @@ rc 1.2 nm, Float32 (SURVEY.md §8d C2-(ii): FCC + jitter, 90 K, dt 2 fs).
           the GPU arm's list radius, threaded pair loop with per-thread force copies) on the same workload, bounded sample.
   workloads  (default run only) the other configurations BASELINE.json names, shorter runs, same fields: c3 = 6mrr
           (replicas when N > 1: its box does not shard), c4 = 1M-atom LJ fluid (decomposed like c2 when N > 1).
+  --dump-outputs DIR  after the timed steps of each workload <w>, the coordinates and velocities a caller of simulate()
+          holds (float32, every atom) are written to DIR/<w>_coords.npy and DIR/<w>_velocities.npy. The inputs are seeded,
+          so two builds run with the same arguments can be compared output for output (c2 and c4 repeat bit for bit on a B200;
+          c3 does not: two runs of the default line differed by up to 3.4e-4 nm after its 40 + 400 steps).
   N > 1   spatial decomposition of ONE system (strong scaling); roofline / fp32 use the per-rank share of bytes and pairs
           and the slowest rank's kernel time.
 
@@ -215,6 +219,8 @@ def main():
     ap.add_argument("--no-cm", action="store_true", help="diagnostic: remove_CM_motion=false")
     ap.add_argument("--replicas", action="store_true", help="N>1: independent replicas instead of the spatial decomposition")
     ap.add_argument("--no-extra", action="store_true", help="only the primary workload (no `workloads` object)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write each workload's coordinates and velocities after its timed steps to DIR/<workload>_<name>.npy")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -228,6 +234,8 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the GPU arm's outputs; the reference arm keeps no state to dump")
         sd, inters, ointers, dt, rc, label = workload(wl, dtype)
         steps = args.steps if args.steps is not None else (10 if wl != "c3" else 100)
         steps = min(steps, 20 if wl == "c2" else (10 if wl == "c4" else 60))  # bounded sample ...
@@ -339,6 +347,10 @@ def run_ours(wl, args, ctx, steps, warmup, with_cpu, with_e2e, brief=False):
     t_ms = max_over_ranks(ev0.elapsed_time(ev1))
     clocks = sampler.stop() if rank == 0 else None
     st1 = sysm.stats()
+    if args.dump_outputs and rank == 0:  # before the profiled run below advances the state
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in (("coords", xs), ("velocities", vs)):
+            np.save(os.path.join(args.dump_outputs, f"{wl}_{name}.npy"), t.cpu().numpy())
     # decomposed: all ranks advance ONE system; replicas: every rank advances its own copy
     mult = 1 if decomposed or world == 1 else world
     value = mult * steps / (t_ms * 1e-3)

@@ -1,10 +1,13 @@
-"""Generate tests/golden/*.npz from the reference's own data files (build container only).
+"""Generate tests/golden/*.npz from the reference's own data files.
 
-Reads /root/reference/data (never available on the GPU box) and writes small
-fixtures: the 6mrr system (per-atom parameters, exclusions, 1-4 specials derived
-by oracle/ffreader.py) and the OpenMM golden forces/energies the reference's
-test/protein.jl:206-276 compares against, plus per-pair literals.
-Usage: python oracle/make_golden.py
+Reads the `data/` directory of a Molly.jl checkout and writes small fixtures: the
+6mrr system (per-atom parameters, exclusions, 1-4 specials derived by
+oracle/ffreader.py) and the OpenMM golden forces/energies the reference's
+test/protein.jl:206-276 compares against, plus per-pair literals. The per-atom
+OpenMM arrays (forces, the state after 100 steps) are kept for a fixed, seeded
+sample of OPENMM_SAMPLE atoms, listed in `openmm_sample`, so that the fixture
+stays under 1 MB; the energies cover the whole system.
+Usage: python oracle/make_golden.py <Molly.jl>/data
 """
 import os
 import sys
@@ -14,23 +17,22 @@ import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import ffreader as fr  # noqa: E402
 
-REF = "/root/reference/data"
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+OPENMM_SAMPLE = 1024
 
 
-def main():
+def main(ref):
     os.makedirs(OUT, exist_ok=True)
-    ff = fr.read_force_field(f"{REF}/force_fields/ff99SBildn.xml", f"{REF}/force_fields/tip3p_standard.xml")
-    atoms, box = fr.read_pdb(f"{REF}/6mrr_equil.pdb")
+    ff = fr.read_force_field(f"{ref}/force_fields/ff99SBildn.xml", f"{ref}/force_fields/tip3p_standard.xml")
+    atoms, box = fr.read_pdb(f"{ref}/6mrr_equil.pdb")
     top = fr.build_topology(atoms, ff)
     coords = np.array([a.xyz for a in atoms], np.float64)
-    amber = f"{REF}/openmm_6mrr/amber"
+    amber = f"{ref}/openmm_6mrr/amber"
     out = dict(
         box=box, coords=coords, mass=top["mass"], charge=top["charge"], sigma=top["sigma"], eps=top["eps"],
-        excluded=top["excluded"], special=top["special"], bonds=top["bonds"], angles=top["angles"],
-        torsions=top["torsions"],
+        excluded=top["excluded"], special=top["special"],
         lj14scale=np.float64(ff.lj14scale), coulomb14scale=np.float64(ff.coulomb14scale),
-        velocities_300K=np.loadtxt(f"{REF}/openmm_6mrr/velocities_300K.txt"),
+        velocities_300K=np.loadtxt(f"{ref}/openmm_6mrr/velocities_300K.txt"),
     )
     for key in ("bond_idx", "bond_par", "angle_idx", "angle_par", "proper_idx", "proper_par", "improper_idx", "improper_par"):
         out[key] = top[key]
@@ -41,17 +43,21 @@ def main():
     # 100 VelocityVerlet steps of the :pme system from velocities_300K (test/protein.jl:277-299: 1e-10 nm, 1e-7 nm/ps)
     out["coordinates_100steps"] = np.loadtxt(f"{amber}/coordinates_100steps.txt")
     out["velocities_100steps"] = np.loadtxt(f"{amber}/velocities_100steps.txt")
+    sample = np.sort(np.random.default_rng(0).choice(len(coords), OPENMM_SAMPLE, replace=False)).astype(np.int32)
+    for key in [k for k in out if k.startswith("forces_")] + ["coordinates_100steps", "velocities_100steps"]:
+        out[key] = out[key][sample]
+    out["openmm_sample"] = sample
     np.savez_compressed(os.path.join(OUT, "6mrr.npz"), **out)
     print("wrote", os.path.join(OUT, "6mrr.npz"), os.path.getsize(os.path.join(OUT, "6mrr.npz")) / 1e6, "MB")
-    water3()
+    water3(ref)
 
 
-def water3():
+def water3(ref):
     """Three TIP3P waters in a 2.0 x 2.1 x 2.2 nm box (data/water_3mol_cubic.pdb), electrostatics only, dist_cutoff 0.9:
     the OpenMM energies / forces the reference's "Ewald" testset holds as literals (test/interactions.jl:1638-1650 for
     :ewald, :1683-1697 for :pme; tolerances there: 2e-4 kJ/mol, 5e-4 kJ/mol/nm)."""
-    ff = fr.read_force_field(f"{REF}/force_fields/tip3p_standard.xml")
-    atoms, box = fr.read_pdb(f"{REF}/water_3mol_cubic.pdb")
+    ff = fr.read_force_field(f"{ref}/force_fields/tip3p_standard.xml")
+    atoms, box = fr.read_pdb(f"{ref}/water_3mol_cubic.pdb")
     top = fr.build_topology(atoms, ff)
     f_pme = np.array([
         [-72.57603365363543, 5.648072796188359, 101.40821248959712], [17.558243038254187, 4.075128117683555, -37.70060863840432],
@@ -73,4 +79,6 @@ def water3():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        raise SystemExit(__doc__)
+    main(sys.argv[1])

@@ -76,7 +76,7 @@ def test_pme_device_functions_on_host_vs_openmm(hostlib, golden_6mrr):
     f, e, _ = H.make_oracle(sd, inters, dtype=np.float64).forces_allpairs(sd["coords"])
     fb, eb = H.bonded_forces_oracle(g, sd["coords"])
     total = f + fb + f4[:, :3] + fx4[:, :3]
-    assert np.linalg.norm(total - g["forces_all_pme_exact"], axis=1).max() < 1e-7
+    assert np.linalg.norm(total[g["openmm_sample"]] - g["forces_all_pme_exact"], axis=1).max() < 1e-7
     e_tot = e + eb + e_recip + info["e_self"] + e_ex + o.lj_dispersion_correction_energy(g["sigma"], g["eps"], box, 1.0)
     assert abs(e_tot - float(g["energy_all_pme_exact"])) < 1e-5
 
