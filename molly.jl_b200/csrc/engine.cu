@@ -1,289 +1,53 @@
-// engine.cu — host side of libmollyb200: context, parameter digestion, rebuild pipeline driver,
-// kernel dispatch and the C ABI declared in include/mollyb200.h.
+// engine.cu — host side of libmollyb200: Engine<T> (parameter digestion, geometry and capacity choice, the rebuild
+// pipeline driver, force dispatch, the MD step and its CUDA graph, the small reductions) and the C ABI declared in
+// include/mollyb200.h. The other host units are headers included into this one translation unit: host_util.h (errors,
+// status macros, device buffers, timing, the runtime -> template dispatch), dynlib.h (NCCL and cuFFT bound with
+// dlopen), decomp.cuh (slab plan and Decomp<T>, all multi-GPU state and transport), pme_host.cuh (PME plan and
+// PmeHost<T>) and specific.cuh (bonded lists and the LJ dispersion correction). Kernels live in force.cuh, cells.cuh,
+// vv.cuh, bonded.cuh, pme.cuh and peer.cuh.
 //
 // There is deliberately no CPU code path: every entry point needs a CUDA device.
 #include <algorithm>
-#include <map>
+#include <climits>
 #include <memory>
-#include <type_traits>
 
-#include "../../include/mollyb200.h"
-#include "bonded.cuh"
 #include "cells.cuh"
 #include "common.cuh"
+#include "decomp.cuh"
+#include "dynlib.h"
 #include "force.cuh"
+#include "host_util.h"
 #include "pair.cuh"
-#include "pme.cuh"
+#include "pme_host.cuh"
+#include "specific.cuh"
 #include "vv.cuh"
 
 namespace mb {
 
-static thread_local std::string g_last_error;
-static int set_error(int code, const std::string& msg) {
-    g_last_error = msg;
-    return code;
+// Kernel variants, as lists for dispatch(). The brick force kernel additionally has UNIFORM = true for COUL_NONE only.
+// Experiment builds (-DMB_EXP_FAST, profiles/r02_experiments.md) instantiate only the LJ and LJ + CRF brick kernels with
+// plain cutoffs, and only in f32 (mb_ctx_create).
+using AllCoulKinds = Vals<COUL_NONE, COUL_PLAIN, COUL_CRF, COUL_EWALD>;
+using AllCutModes = Vals<CUTM_PLAIN, CUTM_SHIFTED, CUTM_TWO_POINT>;
+#ifdef MB_EXP_FAST
+using BrickCoulKinds = Vals<COUL_NONE, COUL_CRF>;
+using BrickCutModes = Vals<CUTM_PLAIN>;
+#else
+using BrickCoulKinds = AllCoulKinds;
+using BrickCutModes = AllCutModes;
+#endif
+
+// Environment switches (diagnostics and tuning aids, INTEGRATION.md), read once when a context is created.
+static bool env_starts(const char* name, char c) {
+    const char* e = getenv(name);
+    return e && e[0] == c;
 }
-
-#define MB_CUDA(call)                                                                                  \
-    do {                                                                                               \
-        cudaError_t err__ = (call);                                                                    \
-        if (err__ != cudaSuccess) {                                                                    \
-            return set_error(MB_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(err__) + " (" + \
-                                              __FILE__ + ":" + std::to_string(__LINE__) + ")");        \
-        }                                                                                              \
-    } while (0)
-#define MB_TRY(expr)                 \
-    do {                             \
-        int rc__ = (expr);           \
-        if (rc__ != MB_OK) return rc__; \
-    } while (0)
-
-struct DevBuf {
-    void* p = nullptr;
-    size_t bytes = 0;
-    ~DevBuf() { release(); }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        bytes = 0;
-    }
-    cudaError_t ensure(size_t nbytes) {
-        if (nbytes <= bytes) return cudaSuccess;
-        release();
-        cudaError_t e = cudaMalloc(&p, nbytes);
-        if (e == cudaSuccess) bytes = nbytes;
-        return e;
-    }
-    template <typename U>
-    U* as() const {
-        return reinterpret_cast<U*>(p);
-    }
+struct EnvSwitches {
+    bool graph = !env_starts("MOLLYB200_NO_GRAPH", '1');             // else the plain-stream MD step
+    bool static_sched = env_starts("MOLLYB200_STATIC_SCHED", '1');   // force kernel takes bricks round-robin, not by ticket
+    bool p2p = !env_starts("MOLLYB200_P2P", '0');                    // else the NCCL transport for decomposed runs
+    int max_nbuf = getenv("MOLLYB200_NBUF") ? atoi(getenv("MOLLYB200_NBUF")) : INT_MAX;  // cap on the force kernel's ring
 };
-
-static bool is_device_ptr(const void* p) {
-    if (!p) return false;
-    cudaPointerAttributes a;
-    cudaError_t e = cudaPointerGetAttributes(&a, p);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return false;
-    }
-    return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
-}
-
-// Optional per-category device timing with CUDA events on the engine's stream (mb_set_profiling).
-struct Prof {
-    enum { FORCE = 0, VV = 1, REBUILD = 2, NCAT = 3 };
-    bool enabled = false;
-    cudaStream_t stream = nullptr;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[NCAT];
-    size_t used[NCAT] = {0, 0, 0};
-    double ms[NCAT] = {0, 0, 0};
-    long long count[NCAT] = {0, 0, 0};
-    ~Prof() {
-        for (int c = 0; c < NCAT; c++)
-            for (auto& p : ev[c]) { cudaEventDestroy(p.first); cudaEventDestroy(p.second); }
-    }
-    void begin(int c) {
-        if (!enabled) return;
-        if (used[c] == ev[c].size()) {
-            if (ev[c].size() >= 8192) { collect(); }
-            if (used[c] == ev[c].size()) {
-                cudaEvent_t a, b;
-                cudaEventCreate(&a);
-                cudaEventCreate(&b);
-                ev[c].emplace_back(a, b);
-            }
-        }
-        cudaEventRecord(ev[c][used[c]].first, stream);
-    }
-    void end(int c) {
-        if (!enabled) return;
-        cudaEventRecord(ev[c][used[c]].second, stream);
-        used[c]++;
-    }
-    void collect() {
-        cudaStreamSynchronize(stream);
-        for (int c = 0; c < NCAT; c++) {
-            for (size_t k = 0; k < used[c]; k++) {
-                float t = 0;
-                if (cudaEventElapsedTime(&t, ev[c][k].first, ev[c][k].second) == cudaSuccess) { ms[c] += t; count[c]++; }
-            }
-            used[c] = 0;
-        }
-    }
-    void reset() {
-        collect();
-        for (int c = 0; c < NCAT; c++) { ms[c] = 0; count[c] = 0; }
-    }
-};
-
-// ---------------------------------------------------------------------------------------------
-// NCCL, bound at run time (dlopen) so that single-GPU users do not need the library. Only what the
-// decomposed step uses: point-to-point halo exchange, grouped broadcasts, one tiny all-reduce.
-// ---------------------------------------------------------------------------------------------
-#include <dlfcn.h>
-extern "C" {
-typedef struct ncclComm* ncclComm_t;
-typedef struct { char internal[128]; } ncclUniqueId;
-typedef enum { ncclSuccess = 0 } ncclResult_t;
-typedef enum { ncclInt8 = 0, ncclChar = 0, ncclFloat64 = 8, ncclDouble = 8 } ncclDataType_t;
-typedef enum { ncclSum = 0 } ncclRedOp_t;
-}
-struct Nccl {
-    void* lib = nullptr;
-    ncclResult_t (*GetUniqueId)(ncclUniqueId*) = nullptr;
-    ncclResult_t (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int) = nullptr;
-    ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
-    ncclResult_t (*GroupStart)() = nullptr;
-    ncclResult_t (*GroupEnd)() = nullptr;
-    ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*Recv)(void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*Broadcast)(const void*, void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
-    const char* (*GetErrorString)(ncclResult_t) = nullptr;
-    bool load() {
-        if (lib) return true;
-        lib = dlopen("libnccl.so.2", RTLD_NOW | RTLD_GLOBAL);
-        if (!lib) lib = dlopen("libnccl.so", RTLD_NOW | RTLD_GLOBAL);
-        if (!lib) return false;
-#define MB_SYM(field, name) field = reinterpret_cast<decltype(field)>(dlsym(lib, name)); if (!field) return false
-        MB_SYM(GetUniqueId, "ncclGetUniqueId");
-        MB_SYM(CommInitRank, "ncclCommInitRank");
-        MB_SYM(CommDestroy, "ncclCommDestroy");
-        MB_SYM(GroupStart, "ncclGroupStart");
-        MB_SYM(GroupEnd, "ncclGroupEnd");
-        MB_SYM(Send, "ncclSend");
-        MB_SYM(Recv, "ncclRecv");
-        MB_SYM(Broadcast, "ncclBroadcast");
-        MB_SYM(AllReduce, "ncclAllReduce");
-        MB_SYM(AllGather, "ncclAllGather");
-        MB_SYM(GetErrorString, "ncclGetErrorString");
-#undef MB_SYM
-        return true;
-    }
-};
-static Nccl g_nccl;
-
-// cuFFT, bound at run time like NCCL (only PME systems need it). Plain library FFT: the spreading, convolution and
-// interpolation kernels around it are ours (pme.cuh).
-struct Cufft {
-    void* lib = nullptr;
-    int (*Plan3d)(int*, int, int, int, int) = nullptr;
-    int (*SetStream)(int, cudaStream_t) = nullptr;
-    int (*ExecC2C)(int, void*, void*, int) = nullptr;
-    int (*ExecZ2Z)(int, void*, void*, int) = nullptr;
-    int (*Destroy)(int) = nullptr;
-    bool load() {
-        if (lib) return true;
-        lib = dlopen("libcufft.so.11", RTLD_NOW | RTLD_GLOBAL);
-        if (!lib) lib = dlopen("libcufft.so", RTLD_NOW | RTLD_GLOBAL);
-        if (!lib) return false;
-#define MB_SYM(field, name) field = reinterpret_cast<decltype(field)>(dlsym(lib, name)); if (!field) return false
-        MB_SYM(Plan3d, "cufftPlan3d");
-        MB_SYM(SetStream, "cufftSetStream");
-        MB_SYM(ExecC2C, "cufftExecC2C");
-        MB_SYM(ExecZ2Z, "cufftExecZ2Z");
-        MB_SYM(Destroy, "cufftDestroy");
-#undef MB_SYM
-        return true;
-    }
-};
-static Cufft g_cufft;
-#define MB_NCCL(call)                                                                                       \
-    do {                                                                                                    \
-        ncclResult_t r__ = (call);                                                                          \
-        if (r__ != ncclSuccess)                                                                             \
-            return set_error(MB_ERR_CUDA, std::string(#call) + ": " + g_nccl.GetErrorString(r__));          \
-    } while (0)
-
-// ---------------------------------------------------------------------------------------------
-// Slab decomposition plan (pure host logic, exported as mb_decomp_plan so it can be tested without a GPU):
-// rank q owns cell layers [q*ncz/P, (q+1)*ncz/P); it needs the h layers below and above its slab (periodic).
-// Segments are contiguous slot ranges [start, start+count) taken from layer_start (ncz + 1 prefix offsets).
-// Both ends enumerate the segments of a (sender, receiver) pair in the receiver's order, so the grouped
-// ncclSend/ncclRecv calls match up.
-// ---------------------------------------------------------------------------------------------
-struct DecompSeg { int peer, start, count; };
-static inline int decomp_layer_lo(int q, int ncz, int nranks) { return (int)(((long long)q * ncz) / nranks); }
-static inline int decomp_layer_owner(int layer, int ncz, int nranks) {
-    for (int q = 0; q < nranks; q++)
-        if (layer >= decomp_layer_lo(q, ncz, nranks) && layer < decomp_layer_lo(q + 1, ncz, nranks)) return q;
-    return nranks - 1;
-}
-static void decomp_needed(int q, int ncz, int h, int nranks, std::vector<int>& out) {
-    out.clear();
-    const int lo = decomp_layer_lo(q, ncz, nranks), hi = decomp_layer_lo(q + 1, ncz, nranks);
-    std::vector<char> seen(ncz, 0);
-    for (int l = lo; l < hi; l++) seen[l] = 1;
-    for (int l = lo - h; l < lo; l++) { int w = ((l % ncz) + ncz) % ncz; if (!seen[w]) { seen[w] = 1; out.push_back(w); } }
-    for (int l = hi; l < hi + h; l++) { int w = l % ncz; if (!seen[w]) { seen[w] = 1; out.push_back(w); } }
-}
-static void decomp_plan(int ncz, int h, int nranks, int rank, const int* layer_start, std::vector<DecompSeg>& send,
-                        std::vector<DecompSeg>& recv) {
-    auto add = [&](std::vector<DecompSeg>& v, int peer, int layer) {
-        int st = layer_start[layer], cnt = layer_start[layer + 1] - st;
-        if (!v.empty() && v.back().peer == peer && v.back().start + v.back().count == st) v.back().count += cnt;
-        else v.push_back({peer, st, cnt});
-    };
-    send.clear();
-    recv.clear();
-    std::vector<int> need;
-    decomp_needed(rank, ncz, h, nranks, need);
-    for (int l : need) add(recv, decomp_layer_owner(l, ncz, nranks), l);
-    for (int q = 0; q < nranks; q++) {
-        if (q == rank) continue;
-        decomp_needed(q, ncz, h, nranks, need);
-        for (int l : need)
-            if (decomp_layer_owner(l, ncz, nranks) == rank) add(send, q, l);
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// PME plan (pure host logic, exported as mb_pme_plan so it is tested on the CPU against oracle/pme.py):
-// alpha = sqrt(-ln(2 tol)) / rc (ewald.jl:373), mesh dims = max(6, ceil(2 alpha L / (3 tol^0.2))) (:484-487),
-// B-spline moduli (:311-361).
-// ---------------------------------------------------------------------------------------------
-static void pme_plan_host(const double box[3], double r_cut, double error_tol, int order, double* alpha_out, int K[3],
-                          std::vector<double> moduli[3]) {
-    const double alpha = std::sqrt(-std::log(2.0 * error_tol)) / r_cut;
-    *alpha_out = alpha;
-    for (int d = 0; d < 3; d++) K[d] = std::max((int)std::ceil(2.0 * alpha * box[d] / (3.0 * std::pow(error_tol, 0.2))), 6);
-    std::vector<double> data(order, 0.0);
-    data[0] = 1.0;
-    for (int k = 3; k < order; k++) {
-        const double d = 1.0 / (k - 1.0);
-        data[k - 1] = 0.0;
-        for (int l = 1; l <= k - 2; l++) data[k - l - 1] = d * (l * data[k - l - 2] + (k - l) * data[k - l - 1]);
-        data[0] *= d;
-    }
-    {
-        const double d = 1.0 / (order - 1.0);
-        data[order - 1] = 0.0;
-        for (int l = 1; l <= order - 2; l++) data[order - l - 1] = d * (l * data[order - l - 2] + (order - l) * data[order - l - 1]);
-        data[0] *= d;
-    }
-    const double two_pi = 6.283185307179586476925;
-    for (int d = 0; d < 3; d++) {
-        const int nd = K[d];
-        std::vector<double> bs((size_t)std::max(nd, order + 1), 0.0);
-        std::vector<double>& mod = moduli[d];
-        mod.assign(nd, 0.0);
-        for (int i = 0; i < order; i++) bs[i + 1] = data[i];
-        for (int i = 0; i < nd; i++) {
-            double sc = 0, ss = 0;
-            for (int j = 0; j < nd; j++) {
-                const double arg = two_pi * i * j / nd;
-                sc += bs[j] * std::cos(arg);
-                ss += bs[j] * std::sin(arg);
-            }
-            mod[i] = sc * sc + ss * ss;
-        }
-        for (int i = 0; i < nd; i++)
-            if (mod[i] < 1e-7) mod[i] = 0.5 * (mod[(i - 1 + nd) % nd] + mod[(i + 1) % nd]);
-    }
-}
 
 class EngineBase {
    public:
@@ -320,7 +84,7 @@ class Engine : public EngineBase {
     using T2 = typename VT<T>::T2;
 
    public:
-    Engine(int device, cudaStream_t stream) : device_(device), stream_(stream) {
+    Engine(int device, cudaStream_t stream) : stream_(stream) {
         cudaDeviceProp prop;
         cudaGetDeviceProperties(&prop, device);
         sm_count_ = prop.multiProcessorCount;
@@ -332,16 +96,12 @@ class Engine : public EngineBase {
             if (cudaStreamCreateWithFlags(&stream_, cudaStreamDefault) == cudaSuccess) own_stream_ = true;
             else stream_ = nullptr;
         }
-        prof_.stream = stream_;
-        const char* ng = getenv("MOLLYB200_NO_GRAPH");
-        graph_enabled_ = !(ng && ng[0] == '1');
-        const char* ss = getenv("MOLLYB200_STATIC_SCHED");
-        static_sched_ = ss && ss[0] == '1';
+        prof_.stream = dc_.stream_ = pme_.stream_ = bonded_.stream_ = stream_;
     }
     ~Engine() override {
         destroy_graph();
-        p2p_close();
-        if (pme_plan_ >= 0 && g_cufft.Destroy) g_cufft.Destroy(pme_plan_);
+        dc_.p2p_close();
+        pme_.destroy_plan();
         if (own_stream_) cudaStreamDestroy(stream_);
     }
 
@@ -497,7 +257,6 @@ class Engine : public EngineBase {
         }
         if (!(lpa == 0 || lpa == 8))
             return set_error(MB_ERR_INVALID, "lanes_per_atom must be 0 (default) or 8: the 4- and 16-lane variants were measured slower and removed");
-        lpa_ = lpa ? lpa : 8;
         have_list_ = false;
         dirty_ = true;
         return MB_OK;
@@ -533,13 +292,12 @@ class Engine : public EngineBase {
         }
         const double min_box = std::min(box_[0], std::min(box_[1], box_[2]));
         path_ = (all_nl && r_list_ > 0 && min_box >= 2.5 * r_list_ && n_ >= 64 && !tric_.on) ? 1 : 0;
-        if (tric_.on && (has_lists() || pme_on_))
+        if (tric_.on && has_specific())
             return set_error(MB_ERR_INVALID, "TriclinicBoundary: specific interaction lists and PME are not supported by this engine");
-        if (tric_.on && decomposed()) return set_error(MB_ERR_INVALID, "TriclinicBoundary: not available in decomposed (multi-GPU) runs");
+        if (tric_.on && dc_.decomposed()) return set_error(MB_ERR_INVALID, "TriclinicBoundary: not available in decomposed (multi-GPU) runs");
         if (path_ == 1 && max_rc > r_list_)
             return set_error(MB_ERR_INVALID, "neighbour list radius is smaller than an interaction cutoff");
         skin_ = (path_ == 1) ? (any_nocut_nl ? 0.0 : r_list_ - max_rc) : 0.0;
-        max_rc_ = max_rc;
         P_.has_lj = 0;
         P_.coul_kind = COUL_NONE;
         P_.lj_rc2 = (T)0;
@@ -653,7 +411,6 @@ class Engine : public EngineBase {
         const int vvb = (int)((n_ + VV_THREADS - 1) / VV_THREADS);
         MB_CUDA(d_partial_.ensure((size_t)std::max(vvb, 2048) * 8 * sizeof(double)));
         have_list_ = false;
-        slots_init_ = false;
         dirty_ = false;
         return MB_OK;
     }
@@ -685,7 +442,7 @@ class Engine : public EngineBase {
             vol *= box_[d];
         }
         if ((double)g.nc[0] * g.nc[1] * g.nc[2] > 2.0e8) return set_error(MB_ERR_INVALID, "cell grid too large");
-        if (nranks_ > g.nc[2]) return set_error(MB_ERR_INVALID, "more ranks than cell layers along z");
+        if (dc_.nranks_ > g.nc[2]) return set_error(MB_ERR_INVALID, "more ranks than cell layers along z");
         g.ncells = g.nc[0] * g.nc[1] * g.nc[2];
         g.rlist2 = (T)(r_list_ * r_list_);
         g.skin_half2 = (T)(0.25 * skin_ * skin_);
@@ -695,7 +452,7 @@ class Engine : public EngineBase {
         int best[3] = {1, 1, 1};
         if (user_b_[0] > 0 && user_b_[1] > 0 && user_b_[2] > 0) {
             for (int d = 0; d < 3; d++) best[d] = std::min(user_b_[d], g.nc[d]);
-            if (nranks_ > 1) best[2] = 1;
+            if (dc_.nranks_ > 1) best[2] = 1;
         } else {
             // Cost model in pair-evaluation units. The persistent force kernel keeps two CTAs per SM busy through a ring of
             // stages (one stage = one brick's halo), so a brick costs its pair work plus a staging share per halo atom and a
@@ -709,7 +466,7 @@ class Engine : public EngineBase {
                 for (int by = 1; by <= bx; by++)
                     for (int bz = 1; bz <= by; bz++) {
                         if (bx > g.nc[0] || by > g.nc[1] || bz > g.nc[2]) continue;
-                        if (nranks_ > 1 && bz != 1) continue;  // slabs are whole cell layers
+                        if (dc_.nranks_ > 1 && bz != 1) continue;  // slabs are whole cell layers
                         double halo = (bx + 4.0) * (by + 4.0) * (bz + 4.0) * rho_c * 1.25 + 64;
                         double owned = (double)bx * by * bz * rho_c;
                         double smem = halo * bytes_per_atom + owned * 1.3 * 8.0 + 256;
@@ -768,7 +525,7 @@ class Engine : public EngineBase {
         while (ctas_per_sm > 1 && (sm_total / ctas_per_sm - 1024 - static_bytes) / stage < 1) ctas_per_sm--;
         const size_t budget = (ctas_per_sm > 1) ? sm_total / ctas_per_sm - 1024 - static_bytes : smem_optin_ - static_bytes;
         nbuf = (int)std::min<size_t>(FORCE_MAX_STAGES, std::max<size_t>(1, budget / stage));
-        if (const char* e = getenv("MOLLYB200_NBUF")) nbuf = std::max(1, std::min(nbuf, atoi(e)));  // tuning aid: shallower ring
+        nbuf = std::max(1, std::min(nbuf, env_.max_nbuf));  // MOLLYB200_NBUF: shallower ring
     }
     size_t build_smem_bytes() const {
         return (size_t)g_.halo_cap * (sizeof(T4) + sizeof(int)) + (size_t)((g_.hcells + 3) & ~3) * sizeof(ushort2) +
@@ -808,458 +565,34 @@ class Engine : public EngineBase {
         return MB_OK;
     }
 
-    // ---- specific (bonded) interaction lists: kind 0 bond (k, r0), 1 angle (k, theta0), 2 torsion (periodicity, phase, k)
+    // ---- terms added after the pair kernel: bonded lists and PME (specific.cuh, pme_host.cuh) ----------------------
     int set_specific(int kind, int64_t n, const int32_t* idx, const double* par) override {
-        if (kind < 0 || kind > 2 || n < 0 || (n > 0 && (!idx || !par))) return set_error(MB_ERR_INVALID, "mb_set_specific: bad arguments");
-        if (n_ <= 0) return set_error(MB_ERR_STATE, "mb_set_specific: set atoms first");
-        const int na = kind + 2, np_ = (kind == 2) ? 3 : 2;
-        std::vector<int> hidx((size_t)n * na);
-        std::vector<T> hpar((size_t)n * np_);
-        for (int64_t t = 0; t < n * na; t++) {
-            int a = idx[t] - 1;  // 1-based in, like InteractionList{2,3,4}Atoms (src/types.jl:89-157)
-            if (a < 0 || a >= n_) return set_error(MB_ERR_INVALID, "mb_set_specific: atom index out of bounds");
-            hidx[t] = a;
-        }
-        for (int64_t t = 0; t < n * np_; t++) hpar[t] = (T)par[t];
-        sp_n_[kind] = n;
-        if (n > 0) {
-            MB_CUDA(d_sp_idx_k_[kind].ensure(hidx.size() * sizeof(int)));
-            MB_CUDA(d_sp_par_k_[kind].ensure(hpar.size() * sizeof(T)));
-            MB_CUDA(cudaMemcpy(d_sp_idx_k_[kind].p, hidx.data(), hidx.size() * sizeof(int), cudaMemcpyHostToDevice));
-            MB_CUDA(cudaMemcpy(d_sp_par_k_[kind].p, hpar.data(), hpar.size() * sizeof(T), cudaMemcpyHostToDevice));
-        }
-        int64_t mx = std::max(sp_n_[0], std::max(sp_n_[1], sp_n_[2]));
-        MB_CUDA(d_sp_partial_.ensure((size_t)(3 * ((mx + BONDED_THREADS - 1) / BONDED_THREADS) + 8) * sizeof(double)));
+        MB_TRY(bonded_.set(kind, n, idx, par, n_));
         destroy_graph();  // the step graph bakes the term counts in
         return MB_OK;
     }
-    bool has_lists() const { return sp_n_[0] + sp_n_[1] + sp_n_[2] > 0; }
-    bool has_specific() const { return has_lists() || pme_on_; }  // everything that is added after the pair kernel
-    // add the bonded forces to f4 (slot order on the brick path, original order on the all-pairs path);
-    // with energy: per-kernel partials are summed into d_sp_energy_ (double, device)
+    int set_pme(double r_cut, double error_tol, int order, double eps_r, int64_t n_pairs, const int32_t* pi, const int32_t* pj) override {
+        MB_TRY(pme_.set(r_cut, error_tol, order, eps_r, n_pairs, pi, pj, n_));
+        if (pme_.on_) destroy_graph();  // the captured step does not contain the PME launches
+        return MB_OK;
+    }
+    int set_dispersion(double r_cut) override { return disp_.set(r_cut); }
+    bool has_specific() const { return bonded_.any() || pme_.on_; }  // everything that is added after the pair kernel
+    // add the bonded and PME forces to f4 (slot order on the brick path, original order on the all-pairs path);
+    // with energy: their sum goes to bonded_.energy() (double, device)
     int launch_bonded(bool energy) {
         if (!has_specific()) return MB_OK;
-        MB_CUDA(d_sp_partial_.ensure(64 * sizeof(double)));  // (set_specific sizes it for the lists; PME alone needs it to exist)
         const int* slot_of = (path_ == 1) ? d_inv_orig_.as<int>() : nullptr;
-        BoxT bx;
-        for (int d = 0; d < 3; d++) bx.L[d] = box_[d];
-        if (energy) {
-            MB_CUDA(d_sp_energy_.ensure(sizeof(double)));
-            MB_CUDA(cudaMemsetAsync(d_sp_energy_.p, 0, sizeof(double), stream_));
-        }
-        double* part = d_sp_partial_.as<double>();
-        BondedLists L;
-        int total_blk = 0;
-        for (int kind = 0; kind < 3; kind++) {
-            L.n[kind] = (int)sp_n_[kind];
-            L.nblk[kind] = (L.n[kind] + BONDED_THREADS - 1) / BONDED_THREADS;
-            L.idx[kind] = d_sp_idx_k_[kind].as<int>();
-            L.par[kind] = d_sp_par_k_[kind].p;
-            total_blk += L.nblk[kind];
-        }
-        if (total_blk > 0) {
-            if (energy) bonded_kernel<T, true><<<total_blk, BONDED_THREADS, 0, stream_>>>(L, slot_of, d_pos4_.as<T4>(), d_f4_.as<T4>(), bx, part);
-            else bonded_kernel<T, false><<<total_blk, BONDED_THREADS, 0, stream_>>>(L, slot_of, d_pos4_.as<T4>(), d_f4_.as<T4>(), bx, part);
-            launches_++;
-            if (energy) {
-                sum_partials_kernel<<<1, 256, 0, stream_>>>(total_blk, part, d_sp_energy_.as<double>());
-                launches_++;
-            }
-        }
-        MB_CUDA(cudaGetLastError());
-        if (pme_on_) MB_TRY(launch_pme(energy));
+        MB_TRY(bonded_.launch(energy, slot_of, d_pos4_.as<T4>(), d_f4_.as<T4>(), box_, launches_));
+        if (pme_.on_)
+            MB_TRY(pme_.launch(energy, n_, box_, h_charge_, d_pos4_.as<T4>(), d_f4_.as<T4>(), slot_of, bonded_.energy(), launches_));
         return MB_OK;
-    }
-
-    // ---- PME reciprocal space + Ewald exclusions (pme.cuh; SURVEY.md §8(f)-3) -------------------------------
-    int set_pme(double r_cut, double error_tol, int order, double eps_r, int64_t n_pairs, const int32_t* pi, const int32_t* pj) override {
-        if (order == 0) { pme_on_ = false; return MB_OK; }
-        if (order != PME_ORDER) return set_error(MB_ERR_INVALID, "mb_set_pme: only B-spline order 5 is implemented (the reference's default)");
-        if (!(r_cut > 0) || !(error_tol > 0 && error_tol < 0.5) || !(eps_r > 0) || n_pairs < 0 || (n_pairs > 0 && (!pi || !pj)))
-            return set_error(MB_ERR_INVALID, "mb_set_pme: bad arguments");
-        if (n_ <= 0) return set_error(MB_ERR_STATE, "mb_set_pme: set atoms first");
-        if (!g_cufft.load()) return set_error(MB_ERR_INVALID, "mb_set_pme: libcufft could not be loaded");
-        pme_pairs_.resize((size_t)2 * n_pairs);
-        for (int64_t k = 0; k < n_pairs; k++) {
-            const int a = pi[k] - 1, b = pj[k] - 1;  // 1-based in
-            if (a < 0 || b < 0 || a >= n_ || b >= n_) return set_error(MB_ERR_INVALID, "mb_set_pme: pair index out of bounds");
-            pme_pairs_[2 * k] = a;
-            pme_pairs_[2 * k + 1] = b;
-        }
-        pme_rc_ = r_cut; pme_tol_ = error_tol; pme_epsr_ = eps_r;
-        pme_on_ = true;
-        pme_ready_ = false;
-        destroy_graph();  // the captured step does not contain the PME launches
-        return MB_OK;
-    }
-    // ---- LJDispersionCorrection (general interaction; lennard_jones.jl:163-275) -----------------------------------
-    int set_dispersion(double r_cut) override {
-        if (r_cut < 0) return set_error(MB_ERR_INVALID, "mb_set_lj_dispersion_correction: negative cutoff");
-        disp_rc_ = r_cut;
-        disp_ready_ = false;
-        return MB_OK;
-    }
-    // factor_6 / factor_12 of the constructor (:170-226): means over all i <= j pairs, N (N + 1) / 2 terms, Lorentz sigma
-    // and geometric epsilon without the zero shortcut; accumulated in double, grouped by distinct (sigma, eps)
-    int dispersion_prepare() {
-        if (disp_ready_ || disp_rc_ <= 0) return MB_OK;
-        if (n_ <= 0) return set_error(MB_ERR_STATE, "LJ dispersion correction: atoms not set");
-        std::map<std::pair<double, double>, double> types;
-        for (int64_t i = 0; i < n_; i++) types[{(double)h_sigma_[i], (double)h_eps_raw_[i]}] += 1.0;
-        std::vector<std::pair<std::pair<double, double>, double>> tv(types.begin(), types.end());
-        double s6 = 0, s12 = 0;
-        for (size_t a = 0; a < tv.size(); a++)
-            for (size_t b = a; b < tv.size(); b++) {
-                const double np = (a == b) ? tv[a].second * (tv[a].second + 1.0) / 2.0 : tv[a].second * tv[b].second;
-                const double sig = (tv[a].first.first + tv[b].first.first) / 2.0;
-                const double e = std::sqrt(tv[a].first.second * tv[b].first.second);
-                const double sg6 = sig * sig * sig * sig * sig * sig;
-                s6 += np * e * sg6;
-                s12 += np * e * sg6 * sg6;
-            }
-        const double nd = (double)n_, n_pairs = nd * (nd + 1.0) / 2.0, pi_ = 3.14159265358979323846;
-        const double rc3 = disp_rc_ * disp_rc_ * disp_rc_;
-        disp_f6_ = 8.0 * pi_ * nd * nd * (-(s6 / n_pairs) / (3.0 * rc3));
-        disp_f12_ = 8.0 * pi_ * nd * nd * ((s12 / n_pairs) / (9.0 * rc3 * rc3 * rc3));
-        disp_ready_ = true;
-        return MB_OK;
-    }
-    // grid dimensions, B-spline moduli, plan, self energy: ewald.jl:363-421 (constructor) and :947-956
-    int pme_prepare() {
-        bool same_box = pme_ready_;
-        for (int d = 0; d < 3; d++) same_box = same_box && (pme_g_.L[d] == box_[d]);
-        if (same_box) return MB_OK;
-        std::vector<double> moduli[3];
-        pme_plan_host(box_, pme_rc_, pme_tol_, PME_ORDER, &pme_alpha_, pme_g_.K, moduli);
-        for (int d = 0; d < 3; d++) {
-            pme_g_.L[d] = box_[d];
-            MB_CUDA(d_pme_bsm_[d].ensure(moduli[d].size() * sizeof(double)));
-            MB_CUDA(cudaMemcpy(d_pme_bsm_[d].p, moduli[d].data(), moduli[d].size() * sizeof(double), cudaMemcpyHostToDevice));
-        }
-        const size_t total = (size_t)pme_g_.K[0] * pme_g_.K[1] * pme_g_.K[2];
-        MB_CUDA(d_pme_grid_.ensure(total * sizeof(T2)));
-        const int conv_blk = (int)((total + PME_THREADS - 1) / PME_THREADS);
-        const int ex_blk = (int)((pme_pairs_.size() / 2 + PME_THREADS - 1) / PME_THREADS);
-        MB_CUDA(d_pme_partial_.ensure((size_t)(conv_blk + ex_blk + 8) * sizeof(double)));
-        if (!pme_pairs_.empty()) {
-            MB_CUDA(d_pme_pairs_.ensure(pme_pairs_.size() * sizeof(int)));
-            MB_CUDA(cudaMemcpy(d_pme_pairs_.p, pme_pairs_.data(), pme_pairs_.size() * sizeof(int), cudaMemcpyHostToDevice));
-        }
-        if (pme_plan_ >= 0) { g_cufft.Destroy(pme_plan_); pme_plan_ = -1; }
-        const int type = (sizeof(T) == 4) ? 0x29 /* CUFFT_C2C */ : 0x69 /* CUFFT_Z2Z */;
-        if (g_cufft.Plan3d(&pme_plan_, pme_g_.K[0], pme_g_.K[1], pme_g_.K[2], type) != 0) {
-            pme_plan_ = -1;
-            return set_error(MB_ERR_CUDA, "cufftPlan3d failed");
-        }
-        if (g_cufft.SetStream(pme_plan_, stream_) != 0) return set_error(MB_ERR_CUDA, "cufftSetStream failed");
-        // self and neutralising-background energy (ewald.jl:947-956)
-        double qs = 0, q2 = 0;
-        for (int64_t i = 0; i < n_; i++) { qs += (double)h_charge_[i]; q2 += (double)h_charge_[i] * (double)h_charge_[i]; }
-        const double f_div = pme_ke_ / pme_epsr_;
-        const double V = box_[0] * box_[1] * box_[2];
-        const double pi_ = 3.14159265358979323846;
-        pme_self_e_ = -f_div * q2 * pme_alpha_ / std::sqrt(pi_) - f_div * pi_ * qs * qs / (2.0 * V * pme_alpha_ * pme_alpha_);
-        pme_ready_ = true;
-        return MB_OK;
-    }
-    int launch_pme(bool energy) {
-        MB_TRY(pme_prepare());
-        const int nb = (int)((n_ + PME_THREADS - 1) / PME_THREADS);
-        const size_t total = (size_t)pme_g_.K[0] * pme_g_.K[1] * pme_g_.K[2];
-        const int conv_blk = (int)((total + PME_THREADS - 1) / PME_THREADS);
-        const int n_ex = (int)(pme_pairs_.size() / 2);
-        const int ex_blk = (n_ex + PME_THREADS - 1) / PME_THREADS;
-        const double f_div = pme_ke_ / pme_epsr_;
-        const double pi_ = 3.14159265358979323846;
-        const double factor = pi_ * pi_ / (pme_alpha_ * pme_alpha_);
-        const double boxfactor = pi_ * box_[0] * box_[1] * box_[2];
-        double* part = d_pme_partial_.as<double>();
-        T2* grid = d_pme_grid_.as<T2>();
-        MB_CUDA(cudaMemsetAsync(grid, 0, total * sizeof(T2), stream_));
-        pme_spread_kernel<T><<<nb, PME_THREADS, 0, stream_>>>((int)n_, pme_g_, d_pos4_.as<T4>(), grid);
-        auto fft = [&](int dir) -> int {
-            const int rc = (sizeof(T) == 4) ? g_cufft.ExecC2C(pme_plan_, grid, grid, dir) : g_cufft.ExecZ2Z(pme_plan_, grid, grid, dir);
-            return rc == 0 ? MB_OK : set_error(MB_ERR_CUDA, "cufftExec failed");
-        };
-        MB_TRY(fft(-1));
-        if (energy) pme_conv_kernel<T, true><<<conv_blk, PME_THREADS, 0, stream_>>>(pme_g_, f_div, factor, boxfactor, d_pme_bsm_[0].as<double>(), d_pme_bsm_[1].as<double>(), d_pme_bsm_[2].as<double>(), grid, part);
-        else pme_conv_kernel<T, false><<<conv_blk, PME_THREADS, 0, stream_>>>(pme_g_, f_div, factor, boxfactor, d_pme_bsm_[0].as<double>(), d_pme_bsm_[1].as<double>(), d_pme_bsm_[2].as<double>(), grid, part);
-        MB_TRY(fft(1));
-        pme_interp_kernel<T><<<nb, PME_THREADS, 0, stream_>>>((int)n_, pme_g_, d_pos4_.as<T4>(), grid, d_f4_.as<T4>());
-        launches_ += 3;
-        if (n_ex > 0) {
-            const int* slot_of = (path_ == 1) ? d_inv_orig_.as<int>() : nullptr;
-            if (energy) ewald_exclusion_kernel<T, true><<<ex_blk, PME_THREADS, 0, stream_>>>(n_ex, d_pme_pairs_.as<int>(), slot_of, d_pos4_.as<T4>(), d_f4_.as<T4>(), pme_g_, pme_alpha_, f_div, part + conv_blk);
-            else ewald_exclusion_kernel<T, false><<<ex_blk, PME_THREADS, 0, stream_>>>(n_ex, d_pme_pairs_.as<int>(), slot_of, d_pos4_.as<T4>(), d_f4_.as<T4>(), pme_g_, pme_alpha_, f_div, part + conv_blk);
-            launches_++;
-        }
-        if (energy) {
-            sum_partials_kernel<<<1, 256, 0, stream_>>>(conv_blk + (n_ex > 0 ? ex_blk : 0), part, d_sp_energy_.as<double>());
-            add_const_kernel<<<1, 1, 0, stream_>>>(d_sp_energy_.as<double>(), pme_self_e_);
-            launches_ += 2;
-        }
-        MB_CUDA(cudaGetLastError());
-        return MB_OK;
-    }
-
-    // ---- decomposition helpers --------------------------------------------------------------------------
-    bool decomposed() const { return nranks_ > 1; }
-    int own_brick0() const { return build_nb_ < 0 ? 0 : build_b0_; }
-    int own_nbricks() const { return build_nb_ < 0 ? g_.nbricks : build_nb_; }
-    int layer_lo(int q) const { return decomp_layer_lo(q, g_.nc[2], nranks_); }
-    // slot ranges and halo segments follow from the cell layer offsets of the current sort (host copy)
-    int decomposed_interval() const { return rebuild_every_ > 0 ? rebuild_every_ : auto_every_; }
-    int update_ownership() {
-        own_valid_ = true;
-        const int ncz = g_.nc[2], per_layer = g_.nc[0] * g_.nc[1];
-        layer_start_.resize(ncz + 1);
-        MB_CUDA(d_layer_start_.ensure((size_t)(ncz + 1) * sizeof(int)));
-        MB_CUDA(cudaMemcpy2DAsync(d_layer_start_.p, sizeof(int), d_cell_start_.p, (size_t)per_layer * sizeof(int), sizeof(int),
-                                  (size_t)ncz + 1, cudaMemcpyDeviceToDevice, stream_));
-        MB_CUDA(cudaMemcpyAsync(layer_start_.data(), d_layer_start_.p, (size_t)(ncz + 1) * sizeof(int), cudaMemcpyDeviceToHost, stream_));
-        MB_CUDA(cudaStreamSynchronize(stream_));
-        const int nbxy = g_.nb[0] * g_.nb[1];
-        own_b0_ = layer_lo(rank_) * nbxy;
-        own_nb_ = (layer_lo(rank_ + 1) - layer_lo(rank_)) * nbxy;
-        own_s0_ = layer_start_[layer_lo(rank_)];
-        own_n_ = layer_start_[layer_lo(rank_ + 1)] - own_s0_;
-        decomp_plan(ncz, g_.h, nranks_, rank_, layer_start_.data(), halo_send_, halo_recv_);
-        // The peer-memory transport carries at most MB_MAX_SEG segments / peers per rank. Whether the plan fits must be
-        // the same answer on every rank and every step, so it is evaluated for all ranks on unit-sized layers
-        // (the segment structure depends only on ncz, h and the rank count).
-        if (plan_key_[0] != ncz || plan_key_[1] != g_.h || plan_key_[2] != nranks_) {
-            plan_key_[0] = ncz; plan_key_[1] = g_.h; plan_key_[2] = nranks_;
-            std::vector<int> unit(ncz + 1);
-            for (int l = 0; l <= ncz; l++) unit[l] = l;
-            plan_fits_ = nranks_ <= MB_MAX_RANKS;
-            std::vector<DecompSeg> sd, rv;
-            std::vector<int> a, b;
-            for (int q = 0; q < nranks_ && plan_fits_; q++) {
-                decomp_plan(ncz, g_.h, nranks_, q, unit.data(), sd, rv);
-                distinct_peers(sd, a);
-                distinct_peers(rv, b);
-                if ((int)sd.size() > MB_MAX_SEG || (int)a.size() > MB_MAX_SEG || (int)b.size() > MB_MAX_SEG) plan_fits_ = false;
-            }
-        }
-        return MB_OK;
-    }
-    bool p2p_active() const { return p2p_ && plan_fits_; }
-    // Decomposed runs rebuild at a fixed interval (every rank must take the same branch without a host round trip).
-    // The interval for the NEXT call is derived from the largest displacement any interval of this call reached:
-    // n_next = 0.8 * n * (skin/2) / d_max, agreed between ranks with one max-all-reduce. Violations are still counted.
-    int adapt_interval() {
-        // largest displacement any rebuild interval of this call reached (device) -> max over ranks -> host; the only host
-        // wait is the one the end of the call has anyway
-        float* dbuf = reinterpret_cast<float*>(d_mom_.as<double>() + 7);
-        max_disp_kernel<<<1, 1, 0, stream_>>>(d_ctl_.as<Control>(), dbuf);
-        launches_++;
-        MB_NCCL(g_nccl.AllReduce(dbuf, dbuf, 1, (ncclDataType_t)7 /* ncclFloat32 */, (ncclRedOp_t)2 /* ncclMax */, comm_, stream_));
-        float d2 = 0.f;
-        MB_CUDA(cudaMemcpyAsync(&d2, dbuf, sizeof(float), cudaMemcpyDeviceToHost, stream_));
-        MB_CUDA(cudaStreamSynchronize(stream_));
-        if (d2 > 0.f && skin_ > 0) {
-            // d2 was reached within adapt_span_ steps of a rebuild; displacements grow at most linearly in time
-            double n_next = 0.8 * std::max(adapt_span_, 1) * (0.5 * skin_) / std::sqrt((double)d2);
-            auto_every_ = (int)std::min(400.0, std::max(5.0, std::floor(n_next)));
-        }
-        return MB_OK;
-    }
-    // forward halo exchange of positions (x, y, z, q as 16/32-byte records): grouped NCCL send/recv between slabs
-    int halo_exchange() {
-        MB_NCCL(g_nccl.GroupStart());
-        for (auto& sg : halo_send_)
-            if (sg.count > 0) MB_NCCL(g_nccl.Send(d_pos4_.as<T4>() + sg.start, (size_t)sg.count * sizeof(T4), ncclChar, sg.peer, comm_, stream_));
-        for (auto& sg : halo_recv_)
-            if (sg.count > 0) MB_NCCL(g_nccl.Recv(d_pos4_.as<T4>() + sg.start, (size_t)sg.count * sizeof(T4), ncclChar, sg.peer, comm_, stream_));
-        MB_NCCL(g_nccl.GroupEnd());
-        for (auto& sg : halo_recv_) MB_TRY(ext_fill(sg.start, sg.count));  // received slots -> extended array (+ ghost copies)
-        return MB_OK;
-    }
-    // replicate the owned segments of positions and velocities on every rank (rebuild / export)
-    int allgather_state() {
-        MB_NCCL(g_nccl.GroupStart());
-        for (int q = 0; q < nranks_; q++) {
-            const int st = layer_start_[layer_lo(q)], cnt = layer_start_[layer_lo(q + 1)] - st;
-            if (cnt <= 0) continue;
-            MB_NCCL(g_nccl.Broadcast(d_pos4_.as<T4>() + st, d_pos4_.as<T4>() + st, (size_t)cnt * sizeof(T4), ncclChar, q, comm_, stream_));
-            MB_NCCL(g_nccl.Broadcast(d_vel4_.as<T4>() + st, d_vel4_.as<T4>() + st, (size_t)cnt * sizeof(T4), ncclChar, q, comm_, stream_));
-        }
-        MB_NCCL(g_nccl.GroupEnd());
-        return MB_OK;
-    }
-    // ---- peer-memory transport (peer.cuh) -------------------------------------------------------------------
-    void p2p_close() {
-        for (int r = 0; r < (int)peer_pos_.size(); r++) {
-            if (r == rank_) continue;
-            if (peer_pos_[r]) cudaIpcCloseMemHandle(peer_pos_[r]);
-            if (peer_comm_[r]) cudaIpcCloseMemHandle(peer_comm_[r]);
-        }
-        peer_pos_.clear();
-        peer_comm_.clear();
-        p2p_ = false;
-        p2p_pos_base_ = nullptr;
-    }
-    // Collective: every rank exports its position array and its PeerComm block as CUDA IPC handles, the handles travel
-    // by one ncclAllGather, and every rank maps the others'. Any failure on any rank (no peer access, IPC not permitted
-    // in this container, too many ranks) leaves ALL ranks on the NCCL transport.
-    int p2p_setup() {
-        if (p2p_pos_base_ == d_pos4e_.p && !peer_pos_.empty()) return MB_OK;  // mapping is current
-        p2p_close();
-        p2p_pos_base_ = d_pos4e_.p;
-        peer_pos_.assign(nranks_, nullptr);
-        peer_comm_.assign(nranks_, nullptr);
-        const char* env = getenv("MOLLYB200_P2P");
-        int ok = !(env && env[0] == '0') && nranks_ <= MB_MAX_RANKS;
-        struct Rec { cudaIpcMemHandle_t pos, comm; };
-        static_assert(sizeof(Rec) == 128, "two 64-byte IPC handles");
-        // 2 MiB so the block is an allocation of its own; zeroed before any peer can learn its address
-        MB_CUDA(d_comm_.ensure(2u << 20));
-        MB_CUDA(cudaMemsetAsync(d_comm_.p, 0, sizeof(PeerComm), stream_));
-        const unsigned long long magic = 0x6d62323030ull + (unsigned long long)rank_;
-        MB_CUDA(cudaMemcpyAsync(reinterpret_cast<char*>(d_comm_.p) + offsetof(PeerComm, magic), &magic, sizeof(magic),
-                                cudaMemcpyHostToDevice, stream_));
-        Rec mine;
-        memset(&mine, 0, sizeof(mine));
-        if (ok && cudaIpcGetMemHandle(&mine.pos, d_pos4e_.p) != cudaSuccess) { ok = 0; cudaGetLastError(); }
-        if (ok && cudaIpcGetMemHandle(&mine.comm, d_comm_.p) != cudaSuccess) { ok = 0; cudaGetLastError(); }
-        MB_CUDA(d_ipc_.ensure((size_t)(nranks_ + 1) * sizeof(Rec) + 16));
-        Rec* d_all = d_ipc_.as<Rec>();
-        MB_CUDA(cudaMemcpyAsync(d_all + nranks_, &mine, sizeof(Rec), cudaMemcpyHostToDevice, stream_));
-        MB_NCCL(g_nccl.AllGather(d_all + nranks_, d_all, sizeof(Rec), ncclChar, comm_, stream_));
-        std::vector<Rec> all(nranks_);
-        MB_CUDA(cudaMemcpyAsync(all.data(), d_all, (size_t)nranks_ * sizeof(Rec), cudaMemcpyDeviceToHost, stream_));
-        MB_CUDA(cudaStreamSynchronize(stream_));
-        for (int r = 0; r < nranks_ && ok; r++) {
-            if (r == rank_) { peer_pos_[r] = d_pos4e_.p; peer_comm_[r] = d_comm_.p; continue; }
-            if (cudaIpcOpenMemHandle(&peer_pos_[r], all[r].pos, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess ||
-                cudaIpcOpenMemHandle(&peer_comm_[r], all[r].comm, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) {
-                ok = 0;
-                cudaGetLastError();
-                break;
-            }
-            unsigned long long got = 0;  // the mapping must show the owner's tag
-            if (cudaMemcpy(&got, reinterpret_cast<char*>(peer_comm_[r]) + offsetof(PeerComm, magic), sizeof(got),
-                           cudaMemcpyDeviceToHost) != cudaSuccess || got != 0x6d62323030ull + (unsigned long long)r) {
-                ok = 0;
-                cudaGetLastError();
-            }
-        }
-        // agree: min over ranks
-        float okf = (float)ok;
-        float* dbuf = reinterpret_cast<float*>(reinterpret_cast<char*>(d_ipc_.p) + (size_t)(nranks_ + 1) * sizeof(Rec));
-        MB_CUDA(cudaMemcpyAsync(dbuf, &okf, sizeof(float), cudaMemcpyHostToDevice, stream_));
-        MB_NCCL(g_nccl.AllReduce(dbuf, dbuf, 1, (ncclDataType_t)7 /* ncclFloat32 */, (ncclRedOp_t)3 /* ncclMin */, comm_, stream_));
-        MB_CUDA(cudaMemcpyAsync(&okf, dbuf, sizeof(float), cudaMemcpyDeviceToHost, stream_));
-        MB_CUDA(cudaStreamSynchronize(stream_));
-        if (okf < 0.5f) {
-            void* keep = p2p_pos_base_;
-            p2p_close();
-            p2p_pos_base_ = keep;            // do not retry on every call
-            peer_pos_.assign(nranks_, nullptr);
-            return MB_OK;
-        }
-        p2p_ = true;
-        return MB_OK;
-    }
-    PeerComm* comm_of(int r) const { return reinterpret_cast<PeerComm*>(peer_comm_[r]); }
-    // distinct peers of a segment list, in first-appearance order
-    static void distinct_peers(const std::vector<DecompSeg>& v, std::vector<int>& out) {
-        out.clear();
-        for (auto& sg : v)
-            if (sg.count > 0 && std::find(out.begin(), out.end(), sg.peer) == out.end()) out.push_back(sg.peer);
-    }
-    PeerPush<T> make_push(unsigned long long epoch, bool with_data) const {
-        PeerPush<T> ps;
-        memset(&ps, 0, sizeof(ps));
-        ps.epoch = epoch;
-        std::vector<int> peers;
-        distinct_peers(halo_send_, peers);
-        if (with_data)
-            for (auto& sg : halo_send_) {
-                if (sg.count <= 0) continue;
-                ps.start[ps.n_seg] = sg.start;
-                ps.count[ps.n_seg] = sg.count;
-                ps.dst[ps.n_seg] = reinterpret_cast<T4*>(peer_pos_[sg.peer]);
-                ps.n_seg++;
-            }
-        for (int q : peers) {
-            ps.wait_flag[ps.n_peer] = &comm_of(rank_)->read_epoch[q];
-            ps.signal_flag[ps.n_peer] = &comm_of(q)->halo_epoch[rank_];
-            ps.n_peer++;
-        }
-        return ps;
-    }
-    PeerWait make_wait(unsigned long long epoch) const {
-        PeerWait w;
-        memset(&w, 0, sizeof(w));
-        w.epoch = epoch;
-        std::vector<int> peers;
-        distinct_peers(halo_recv_, peers);
-        for (int q : peers) w.flag[w.n++] = &comm_of(rank_)->halo_epoch[q];
-        return w;
-    }
-    PeerSignal make_signal(unsigned long long epoch, bool with_mom) const {
-        PeerSignal sg;
-        memset(&sg, 0, sizeof(sg));
-        sg.epoch = epoch;
-        std::vector<int> peers;
-        distinct_peers(halo_recv_, peers);
-        for (int q : peers) sg.read_flag[sg.n_peer++] = &comm_of(q)->read_epoch[rank_];
-        if (with_mom) {
-            const int par = (int)(epoch & 1ull);
-            sg.n_mom = nranks_;
-            for (int r = 0; r < nranks_; r++) {
-                sg.mom_dst[r] = comm_of(r)->mom[par][rank_];
-                sg.mom_flag[r] = &comm_of(r)->mom_epoch[par][rank_];
-            }
-        }
-        return sg;
     }
 
     int comm_init(const void* uid, int rank, int nranks) override {
-        if (nranks < 1 || rank < 0 || rank >= nranks || !uid) return set_error(MB_ERR_INVALID, "mb_comm_init: bad arguments");
-        if (!g_nccl.load()) return set_error(MB_ERR_INVALID, "mb_comm_init: libnccl.so.2 could not be loaded");
-        p2p_close();
-        if (comm_) { g_nccl.CommDestroy(comm_); comm_ = nullptr; }
-        rank_ = rank;
-        nranks_ = nranks;
-        if (nranks > 1) {
-            ncclUniqueId id;
-            memcpy(&id, uid, sizeof(id));
-            MB_NCCL(g_nccl.CommInitRank(&comm_, nranks, id, rank));
-            MB_CUDA(d_mom_.ensure(8 * sizeof(double)));
-        }
+        MB_TRY(dc_.comm_init(uid, rank, nranks));
         have_list_ = false;
         dirty_ = true;
-        return MB_OK;
-    }
-
-    // The neighbour list is the one large stream the force kernel re-reads every step (131 MB at C2, larger than what
-    // L2 keeps under plain LRU streaming). Pin a fraction of it in L2 with an access-policy window: lines of the window
-    // are kept "persisting" with probability hitRatio, the rest stream through.
-    int set_l2_persistence() {
-        // opt-in (MOLLYB200_L2PERSIST=1): measured on B200 at C2 it changes nothing (83.8 us without, 84.3-86.2 us with), the
-        // kernel is not bound by the list stream
-        const char* on = getenv("MOLLYB200_L2PERSIST");
-        if (!(on && on[0] == '1')) return MB_OK;
-        int max_persist = 0, max_window = 0;
-        cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, device_);
-        cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, device_);
-        if (max_persist <= 0 || max_window <= 0) return MB_OK;
-        const char* fr = getenv("MOLLYB200_L2PERSIST_FRAC");
-        const double frac = fr ? atof(fr) : 0.75;
-        size_t persist = (size_t)(frac * max_persist);
-        if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, persist) != cudaSuccess) { cudaGetLastError(); return MB_OK; }
-        DevBuf& lst = d_list_;
-        size_t bytes = std::min((size_t)n_ * g_.stride * sizeof(unsigned short), (size_t)max_window);
-        cudaStreamAttrValue attr;
-        memset(&attr, 0, sizeof(attr));
-        attr.accessPolicyWindow.base_ptr = lst.p;
-        attr.accessPolicyWindow.num_bytes = bytes;
-        attr.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)persist / (double)bytes);
-        attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        if (cudaStreamSetAttribute(stream_, cudaStreamAttributeAccessPolicyWindow, &attr) != cudaSuccess) cudaGetLastError();
         return MB_OK;
     }
 
@@ -1267,21 +600,23 @@ class Engine : public EngineBase {
     int launch_build(bool count_only) {
         const size_t smem = build_smem_bytes();
         const bool has_ex = !ex_ptr_.empty() || !sp_ptr_.empty();
-        auto go = [&](auto kern) -> int {
-            MB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            // few bricks (small systems, narrow slabs): several CTAs share a brick's atoms so that the SMs are filled
-            const int split = std::max(1, std::min(4, (4 * sm_count_ + own_nbricks() - 1) / std::max(own_nbricks(), 1)));
-            kern<<<own_nbricks() * split, 256, smem, stream_>>>(d_ctl_.as<Control>(), g_, d_hdrs_.as<BrickHdr>(), d_runs_.as<Run>(),
-                                                     d_irows_.as<IRow>(), d_hcs_.as<ushort2>(), d_pos4e_.as<T4>(), d_orig_e_.as<int>(),
-                                                     ex_ptr_dev(), ex_idx_dev(), sp_ptr_dev(), sp_idx_dev(),
-                                                     count_only ? nullptr : d_list_.as<unsigned short>(),
-                                                     count_only ? nullptr : d_slist_.as<unsigned short>(),
-                                                     count_only ? nullptr : d_counts_.as<ushort2>(),
-                                                     count_only ? nullptr : d_task_tab_.as<int2>(), own_brick0(), split);
-            return MB_OK;
-        };
-        if (count_only) { if (has_ex) MB_TRY(go(build_lists_kernel<T, true, true>)); else MB_TRY(go(build_lists_kernel<T, true, false>)); }
-        else { if (has_ex) MB_TRY(go(build_lists_kernel<T, false, true>)); else MB_TRY(go(build_lists_kernel<T, false, false>)); }
+        MB_TRY(dispatch(count_only, [&](auto COUNT) {
+            return dispatch(has_ex, [&](auto EX) -> int {
+                auto kern = build_lists_kernel<T, COUNT, EX>;
+                MB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                // few bricks (small systems, narrow slabs): several CTAs share a brick's atoms so that the SMs are filled
+                const int nbr = dc_.own_nbricks(g_.nbricks);
+                const int split = std::max(1, std::min(4, (4 * sm_count_ + nbr - 1) / std::max(nbr, 1)));
+                kern<<<nbr * split, 256, smem, stream_>>>(d_ctl_.as<Control>(), g_, d_hdrs_.as<BrickHdr>(), d_runs_.as<Run>(),
+                                                          d_irows_.as<IRow>(), d_hcs_.as<ushort2>(), d_pos4e_.as<T4>(), d_orig_e_.as<int>(),
+                                                          ex_ptr_dev(), ex_idx_dev(), sp_ptr_dev(), sp_idx_dev(),
+                                                          count_only ? nullptr : d_list_.as<unsigned short>(),
+                                                          count_only ? nullptr : d_slist_.as<unsigned short>(),
+                                                          count_only ? nullptr : d_counts_.as<ushort2>(),
+                                                          count_only ? nullptr : d_task_tab_.as<int2>(), dc_.own_brick0(), split);
+                return MB_OK;
+            });
+        }));
         launches_++;
         MB_CUDA(cudaGetLastError());
         return MB_OK;
@@ -1334,6 +669,14 @@ class Engine : public EngineBase {
         return MB_OK;
     }
 
+    // slot-order state in original order from coords (and the charges, LJ parts and masses of prepare())
+    void init_slots(const T* coords_dev) {
+        init_slots_kernel<T><<<(int)((n_ + 255) / 256), 256, 0, stream_>>>((int)n_, coords_dev, d_charge_in_.as<T>(), d_ljp_in_.as<T2>(),
+                                                                        d_mass_in_.as<T>(), d_pos4_.as<T4>(), d_vel4_.as<T4>(),
+                                                                        d_lj2_.as<T2>(), d_orig_.as<int>(), d_inv_orig_.as<int>(),
+                                                                        d_mass_.as<T>(), d_xref4_.as<T4>());
+        launches_++;
+    }
     int read_ctl(Control& c) {
         MB_CUDA(cudaMemcpyAsync(&c, d_ctl_.p, sizeof(Control), cudaMemcpyDeviceToHost, stream_));
         MB_CUDA(cudaStreamSynchronize(stream_));
@@ -1348,24 +691,15 @@ class Engine : public EngineBase {
     // Synchronous first build: derives halo capacity and list stride from the actual configuration.
     // coords_dev: n x 3 device array in original order.
     int first_build(const T* coords_dev) {
-        const int nb = (int)((n_ + 255) / 256);
-        build_nb_ = -1;  // lists for every brick (capacities are global; mb_forces evaluates the whole box)
-        own_valid_ = false;
-        init_slots_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, coords_dev, d_charge_in_.as<T>(), d_ljp_in_.as<T2>(),
-                                                      d_mass_in_.as<T>(), d_pos4_.as<T4>(), d_vel4_.as<T4>(), d_lj2_.as<T2>(),
-                                                      d_orig_.as<int>(), d_inv_orig_.as<int>(), d_mass_.as<T>(), d_xref4_.as<T4>());
-        launches_++;
-        slots_init_ = true;
+        dc_.build_nb_ = -1;  // lists for every brick (capacities are global; mb_forces evaluates the whole box)
+        dc_.own_valid_ = false;
+        init_slots(coords_dev);
         for (int attempt = 0; attempt < 8; attempt++) {
             MB_TRY(choose_geometry());
             MB_TRY(alloc_brick_tables());
             // pass A: sort + tables with unlimited halo capacity to measure
             g_.halo_cap = 65535;
-            g_.stride = 0;
-            g_.sstride = 0;
-            g_.task_cap = 0;
-            g_.ext_cap = 0;
-            g_.ghost_cap = 0;
+            g_.stride = g_.sstride = g_.task_cap = g_.ext_cap = g_.ghost_cap = 0;
             MB_TRY(set_flag_rebuild());
             MB_TRY(enqueue_rebuild(false, true));
             Control c;
@@ -1414,13 +748,11 @@ class Engine : public EngineBase {
             MB_TRY(enqueue_rebuild(true, false));
             MB_TRY(read_ctl(c));
             if (c.overflow) return set_error(MB_ERR_CAPACITY, "neighbour capacity overflow during first build");
-            last_ctl_ = c;
             have_list_ = true;
             geom_version_++;
-            set_l2_persistence();
-            if (decomposed()) {
-                MB_TRY(update_ownership());
-                since_rebuild_ = 0;
+            if (dc_.decomposed()) {
+                MB_TRY(dc_.update_ownership(g_, d_cell_start_.as<int>()));
+                dc_.since_rebuild_ = 0;
             }
             return MB_OK;
         }
@@ -1428,131 +760,135 @@ class Engine : public EngineBase {
     }
 
     // ------------------------------------------------------------------------------------------
-    template <int COUL, bool UNIFORM, int CUTM, bool ENERGY>
-    int launch_force_t(ForceOut<T> out, int brick0, int nbr) {
+    // the brick force kernel `kern` (one variant of brick_force_kernel) over bricks [brick0, brick0 + nbr)
+    template <typename K>
+    int launch_brick_force(K kern, ForceOut<T> out, int brick0, int nbr) {
         int nbuf, per_sm;
         force_shape(nbuf, per_sm);
         const size_t smem = (size_t)nbuf * force_stage();
         const int grid = std::max(1, std::min(nbr, per_sm * sm_count_));
         force_grid_ = grid;
-        auto kern = brick_force_kernel<T, COUL, UNIFORM, CUTM, ENERGY>;
         MB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         prof_.begin(Prof::FORCE);
         kern<<<grid, FORCE_THREADS, smem, stream_>>>(g_, P_, d_hdrs_.as<BrickHdr>(), d_runs_.as<Run>(), d_task_tab_.as<int2>(),
                                                      d_pos4e_.as<T4>(), d_lj2e_.as<T2>(), d_list_.as<unsigned short>(),
                                                      d_slist_.as<unsigned short>(), out, brick0, nbr, nbuf,
-                                                     static_sched_ ? nullptr : d_sched_.as<unsigned int>());
+                                                     env_.static_sched ? nullptr : d_sched_.as<unsigned int>());
         prof_.end(Prof::FORCE);
         launches_++;
         n_force_evals_++;
         MB_CUDA(cudaGetLastError());
         return MB_OK;
     }
-    template <int COUL, bool UNIFORM>
-    int launch_force_c(bool energy, ForceOut<T> out, int b0, int nbr) {
-#ifdef MB_EXP_FAST  // experiment builds (scripts/): only the plain-cutoff variants are instantiated
-        if (cutm_ != CUTM_PLAIN) return set_error(MB_ERR_INVALID, "experiment build: plain cutoffs only");
-#else
-        if (cutm_ == CUTM_TWO_POINT) return energy ? launch_force_t<COUL, UNIFORM, CUTM_TWO_POINT, true>(out, b0, nbr) : launch_force_t<COUL, UNIFORM, CUTM_TWO_POINT, false>(out, b0, nbr);
-        if (cutm_ == CUTM_SHIFTED) return energy ? launch_force_t<COUL, UNIFORM, CUTM_SHIFTED, true>(out, b0, nbr) : launch_force_t<COUL, UNIFORM, CUTM_SHIFTED, false>(out, b0, nbr);
-#endif
-        return energy ? launch_force_t<COUL, UNIFORM, CUTM_PLAIN, true>(out, b0, nbr) : launch_force_t<COUL, UNIFORM, CUTM_PLAIN, false>(out, b0, nbr);
-    }
     // owned_only: in a decomposed run the step loop evaluates only this rank's slab of bricks
     int launch_force(bool energy, bool owned_only = false) {
-        const int b0 = owned_only ? own_b0_ : 0;
-        const int nbr = owned_only ? own_nb_ : g_.nbricks;
+        const int b0 = owned_only ? dc_.own_b0_ : 0;
+        const int nbr = owned_only ? dc_.own_nb_ : g_.nbricks;
         ForceOut<T> out;
         out.f4 = d_f4_.as<T4>();
         out.pe_partial = d_pe_partial_.as<double>();
         out.vir_partial = d_pe_partial_.as<double>() + std::max(g_.nbricks, 4 * sm_count_);
-        out.gate = gate_;  // one-shot: set by the decomposed step in front of this launch
-        memset(&gate_, 0, sizeof(gate_));
-        switch (P_.coul_kind) {
-            case COUL_NONE:
-                return P_.uniform_lj ? launch_force_c<COUL_NONE, true>(energy, out, b0, nbr) : launch_force_c<COUL_NONE, false>(energy, out, b0, nbr);
-#ifndef MB_EXP_FAST
-            case COUL_PLAIN: return launch_force_c<COUL_PLAIN, false>(energy, out, b0, nbr);
-            default: return launch_force_c<COUL_EWALD, false>(energy, out, b0, nbr);
-#else
-            default: return set_error(MB_ERR_INVALID, "experiment build: LJ and LJ + CoulombReactionField only");
-#endif
-            case COUL_CRF: return launch_force_c<COUL_CRF, false>(energy, out, b0, nbr);
-        }
+        out.gate = dc_.gate_;  // one-shot: set by the decomposed step in front of this launch
+        memset(&dc_.gate_, 0, sizeof(dc_.gate_));
+        return dispatch(BrickCoulKinds{}, P_.coul_kind, [&](auto COUL) {
+            return dispatch(BrickCutModes{}, cutm_, [&](auto CUTM) {
+                return dispatch(energy, [&](auto EN) {
+                    if constexpr (COUL == COUL_NONE)
+                        return dispatch(P_.uniform_lj != 0, [&](auto UNI) {
+                            return launch_brick_force(brick_force_kernel<T, COUL, UNI, CUTM, EN>, out, b0, nbr);
+                        });
+                    else
+                        return launch_brick_force(brick_force_kernel<T, COUL, false, CUTM, EN>, out, b0, nbr);
+                });
+            }, "experiment build: plain cutoffs only");
+        }, "experiment build: LJ and LJ + CoulombReactionField only");
     }
 
-    template <int COUL>
-    int launch_allpairs_c(bool energy, const T4* posq, const T2* lj2, T4* f4, int nblk) {
+    // no-list kernel over pos4 / lj2 in original order, forces into f4
+    int launch_allpairs(bool energy) {
+        const int nblk = (int)((n_ + AP_THREADS - 1) / AP_THREADS);
+        MB_CUDA(d_pe_partial_.ensure((size_t)nblk * 7 * sizeof(double)));
         double* pe = d_pe_partial_.as<double>();
         double* vir = pe + nblk;
         T Lx = (T)box_[0], Ly = (T)box_[1], Lz = (T)box_[2];
-#define MB_AP(SH, EN)                                                                                              \
-    allpairs_force_kernel<T, COUL, SH, EN><<<nblk, AP_THREADS, 0, stream_>>>((int)n_, P_, Lx, Ly, Lz, tric_, posq, lj2, \
-                                                                              ex_ptr_dev(), ex_idx_dev(), sp_ptr_dev(), \
-                                                                              sp_idx_dev(), f4, pe, vir)
         prof_.begin(Prof::FORCE);
-        if (cutm_ == CUTM_TWO_POINT) { if (energy) MB_AP(CUTM_TWO_POINT, true); else MB_AP(CUTM_TWO_POINT, false); }
-        else if (cutm_ == CUTM_SHIFTED) { if (energy) MB_AP(CUTM_SHIFTED, true); else MB_AP(CUTM_SHIFTED, false); }
-        else { if (energy) MB_AP(CUTM_PLAIN, true); else MB_AP(CUTM_PLAIN, false); }
+        MB_TRY(dispatch(AllCoulKinds{}, P_.coul_kind, [&](auto COUL) {
+            return dispatch(AllCutModes{}, cutm_, [&](auto CUTM) {
+                return dispatch(energy, [&](auto EN) {
+                    allpairs_force_kernel<T, COUL, CUTM, EN><<<nblk, AP_THREADS, 0, stream_>>>(
+                        (int)n_, P_, Lx, Ly, Lz, tric_, d_pos4_.as<T4>(), d_lj2_.as<T2>(), ex_ptr_dev(), ex_idx_dev(), sp_ptr_dev(), sp_idx_dev(),
+                        d_f4_.as<T4>(), pe, vir);
+                    return MB_OK;
+                });
+            });
+        }));
         prof_.end(Prof::FORCE);
-#undef MB_AP
         launches_++;
         n_force_evals_++;
         MB_CUDA(cudaGetLastError());
         return MB_OK;
     }
-    int launch_allpairs(bool energy, const T4* posq, const T2* lj2, T4* f4) {
-        const int nblk = (int)((n_ + AP_THREADS - 1) / AP_THREADS);
-        MB_CUDA(d_pe_partial_.ensure((size_t)nblk * 7 * sizeof(double)));
-        switch (P_.coul_kind) {
-            case COUL_NONE: return launch_allpairs_c<COUL_NONE>(energy, posq, lj2, f4, nblk);
-            case COUL_PLAIN: return launch_allpairs_c<COUL_PLAIN>(energy, posq, lj2, f4, nblk);
-            case COUL_CRF: return launch_allpairs_c<COUL_CRF>(energy, posq, lj2, f4, nblk);
-            default: return launch_allpairs_c<COUL_EWALD>(energy, posq, lj2, f4, nblk);
-        }
-    }
 
     // host/device argument views ----------------------------------------------------------------
-    // returns a device pointer holding `count` T values of `user` (copying if user is a host pointer)
-    int view_in(const void* user, size_t count, DevBuf& stage, const T** out) {
-        if (!user) { *out = nullptr; return MB_OK; }
-        if (is_device_ptr(user)) { *out = reinterpret_cast<const T*>(user); return MB_OK; }
+    // device pointer for `count` T outputs to `user`: user itself if it is device memory, else the staging buffer, which
+    // view_out_done copies back; `load` fills the stage with user's values first (in-out arguments, outputs added to)
+    int view_out(void* user, size_t count, DevBuf& stage, bool load, T** out) {
+        if (!user || is_device_ptr(user)) { *out = reinterpret_cast<T*>(user); return MB_OK; }
         MB_CUDA(stage.ensure(count * sizeof(T)));
-        MB_CUDA(cudaMemcpyAsync(stage.p, user, count * sizeof(T), cudaMemcpyHostToDevice, stream_));
+        if (load) MB_CUDA(cudaMemcpyAsync(stage.p, user, count * sizeof(T), cudaMemcpyHostToDevice, stream_));
         *out = stage.as<T>();
+        return MB_OK;
+    }
+    int view_out_done(void* user, const T* dev, size_t count) {
+        if (dev != user) MB_CUDA(cudaMemcpyAsync(user, dev, count * sizeof(T), cudaMemcpyDeviceToHost, stream_));
+        return MB_OK;
+    }
+    // device pointer holding `count` T values of `user` (copied if user is a host pointer)
+    int view_in(const void* user, size_t count, DevBuf& stage, const T** out) {
+        T* p = nullptr;
+        MB_TRY(view_out(const_cast<void*>(user), count, stage, true, &p));
+        *out = p;
+        return MB_OK;
+    }
+    // per-block partial sums of a velocity reduction (kern writes k doubles per 256-thread block) -> s[0..k) on the host
+    int reduce_to_host(void (*kern)(int, const T*, const T*, double*), const T* vels, int k, double* s) {
+        const int nb = (int)((n_ + 255) / 256);
+        MB_CUDA(d_partial_.ensure((size_t)nb * k * sizeof(double)));
+        kern<<<nb, 256, 0, stream_>>>((int)n_, vels, d_mass_in_.as<T>(), d_partial_.as<double>());
+        launches_++;
+        std::vector<double> part((size_t)nb * k);
+        MB_CUDA(cudaMemcpyAsync(part.data(), d_partial_.p, part.size() * sizeof(double), cudaMemcpyDeviceToHost, stream_));
+        MB_CUDA(cudaStreamSynchronize(stream_));
+        for (int d = 0; d < k; d++) s[d] = 0;
+        for (int b = 0; b < nb; b++) for (int d = 0; d < k; d++) s[d] += part[(size_t)k * b + d];
         return MB_OK;
     }
 
     // ------------------------------------------------------------------------------------------
     // make the slot-order state reflect `coords` (and vels), rebuilding the list when required
     int sync_state_from(const T* coords_dev, const T* vels_dev) {
-        const int nb = (int)((n_ + 255) / 256);
-        if (!have_list_) {
-            MB_TRY(first_build(coords_dev));
-            if (vels_dev) {
-                ingest_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, g_, coords_dev, vels_dev, d_orig_.as<int>(), d_xref4_.as<T4>(),
-                                                          d_pos4_.as<T4>(), d_vel4_.as<T4>(), &d_ctl_.as<Control>()->disp);
-                launches_++;
-                MB_TRY(ext_fill(0, (int)n_));
-            }
-            return MB_OK;
-        }
-        ingest_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, g_, coords_dev, vels_dev, d_orig_.as<int>(), d_xref4_.as<T4>(),
-                                                  d_pos4_.as<T4>(), d_vel4_.as<T4>(), &d_ctl_.as<Control>()->rebuild);
+        const bool first = !have_list_;
+        if (first) MB_TRY(first_build(coords_dev));
+        if (first && !vels_dev) return MB_OK;
+        // right after a first build the displacement check reports into ctl->disp instead of requesting a rebuild
+        ingest_kernel<T><<<(int)((n_ + 255) / 256), 256, 0, stream_>>>((int)n_, g_, coords_dev, vels_dev, d_orig_.as<int>(),
+                                                                    d_xref4_.as<T4>(), d_pos4_.as<T4>(), d_vel4_.as<T4>(),
+                                                                    first ? &d_ctl_.as<Control>()->disp : &d_ctl_.as<Control>()->rebuild);
         launches_++;
-        if (decomposed()) {
+        if (first) return ext_fill(0, (int)n_);
+        if (dc_.decomposed()) {
             // Every rank holds the full state here. The lists of the previous call stay valid until an atom has moved more
             // than skin/2 from its position at the last rebuild (ingest_kernel just checked that on identical data on every
             // rank) or the rebuild interval has run out; the host needs the answer because ownership follows from the sort.
             int flag = 0;
             MB_CUDA(cudaMemcpyAsync(&flag, &d_ctl_.as<Control>()->rebuild, sizeof(int), cudaMemcpyDeviceToHost, stream_));
             MB_CUDA(cudaStreamSynchronize(stream_));
-            if (flag || !own_valid_ || since_rebuild_ >= decomposed_interval()) {
-                if (own_valid_) { build_b0_ = own_b0_; build_nb_ = own_nb_; }  // lists only for the owned slab
+            if (flag || !dc_.own_valid_ || dc_.since_rebuild_ >= dc_.interval(rebuild_every_)) {
+                if (dc_.own_valid_) { dc_.build_b0_ = dc_.own_b0_; dc_.build_nb_ = dc_.own_nb_; }  // lists only for the owned slab
                 MB_TRY(set_flag_rebuild());
                 MB_TRY(enqueue_rebuild(true, false));
-                MB_TRY(update_ownership());
-                since_rebuild_ = 0;
+                MB_TRY(dc_.update_ownership(g_, d_cell_start_.as<int>()));
+                dc_.since_rebuild_ = 0;
             } else {
                 MB_TRY(ext_fill(0, (int)n_));
             }
@@ -1563,10 +899,15 @@ class Engine : public EngineBase {
         return MB_OK;
     }
 
-    int check_overflow_sync() {
+    // end of a call: on the brick path read back the capacity flags (a host wait), else just wait
+    int finish_call() {
+        MB_CUDA(cudaGetLastError());
+        if (path_ == 0) {
+            MB_CUDA(cudaStreamSynchronize(stream_));
+            return MB_OK;
+        }
         Control c;
         MB_TRY(read_ctl(c));
-        last_ctl_ = c;
         if (c.overflow) {
             have_list_ = false;  // next call re-derives capacities
             static const int zero = 0;
@@ -1588,15 +929,11 @@ class Engine : public EngineBase {
         int n_partials = 0;
         const int* orig = nullptr;
         if (path_ == 0) {
-            // original order; posq packed into pos4
-            init_slots_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, xc, d_charge_in_.as<T>(), d_ljp_in_.as<T2>(), d_mass_in_.as<T>(),
-                                                          d_pos4_.as<T4>(), d_vel4_.as<T4>(), d_lj2_.as<T2>(), d_orig_.as<int>(),
-                                                          d_inv_orig_.as<int>(), d_mass_.as<T>(), d_xref4_.as<T4>());
-            launches_++;
-            MB_TRY(launch_allpairs(energy, d_pos4_.as<T4>(), d_lj2_.as<T2>(), d_f4_.as<T4>()));
+            init_slots(xc);  // original order; posq packed into pos4
+            MB_TRY(launch_allpairs(energy));
             n_partials = (int)((n_ + AP_THREADS - 1) / AP_THREADS);
         } else {
-            if (decomposed()) have_list_ = false;  // forces()/potential_energy() evaluate the whole box on every rank
+            if (dc_.decomposed()) have_list_ = false;  // forces()/potential_energy() evaluate the whole box on every rank
             MB_TRY(sync_state_from(xc, nullptr));
             MB_TRY(launch_force(energy));
             n_partials = force_grid_;
@@ -1605,16 +942,11 @@ class Engine : public EngineBase {
         if (with_specific) MB_TRY(launch_bonded(pe != nullptr));
         // outputs (ADD semantics)
         if (fs) {
-            if (is_device_ptr(fs)) {
-                scatter_forces_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, d_f4_.as<T4>(), orig, reinterpret_cast<T*>(fs));
-                launches_++;
-            } else {
-                MB_CUDA(d_stage_b_.ensure(3 * (size_t)n_ * sizeof(T)));
-                MB_CUDA(cudaMemcpyAsync(d_stage_b_.p, fs, 3 * (size_t)n_ * sizeof(T), cudaMemcpyHostToDevice, stream_));
-                scatter_forces_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, d_f4_.as<T4>(), orig, d_stage_b_.as<T>());
-                launches_++;
-                MB_CUDA(cudaMemcpyAsync(fs, d_stage_b_.p, 3 * (size_t)n_ * sizeof(T), cudaMemcpyDeviceToHost, stream_));
-            }
+            T* fo = nullptr;
+            MB_TRY(view_out(fs, 3 * (size_t)n_, d_stage_b_, true, &fo));
+            scatter_forces_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, d_f4_.as<T4>(), orig, fo);
+            launches_++;
+            MB_TRY(view_out_done(fs, fo, 3 * (size_t)n_));
         }
         if (energy) {
             // stage scalars on device: [pe, vir(9)]
@@ -1638,13 +970,13 @@ class Engine : public EngineBase {
             reduce_partials_kernel<T><<<1, 256, 0, stream_>>>(n_partials, pp, vp, pe_target, vir_target, nullptr);
             launches_++;
             if (with_specific && has_specific() && pe_target) {
-                add_double_kernel<T><<<1, 1, 0, stream_>>>(d_sp_energy_.as<double>(), pe_target);
+                add_double_kernel<T><<<1, 1, 0, stream_>>>(bonded_.energy(), pe_target);
                 launches_++;
             }
-            if (with_specific && disp_rc_ > 0) {  // LJDispersionCorrection: E = (f6 + f12) / V; virial 2 U6 + 4 U12 on the diagonal
-                MB_TRY(dispersion_prepare());
+            if (with_specific && disp_.rc_ > 0) {  // LJDispersionCorrection: E = (f6 + f12) / V; virial 2 U6 + 4 U12 on the diagonal
+                MB_TRY(disp_.prepare(n_, h_sigma_, h_eps_raw_));
                 const double vol = box_[0] * box_[1] * box_[2];
-                const double u6 = disp_f6_ / vol, u12 = disp_f12_ / vol;
+                const double u6 = disp_.f6_ / vol, u12 = disp_.f12_ / vol;
                 add_scalars_kernel<T><<<1, 1, 0, stream_>>>(pe_target, (T)(u6 + u12), vir_target, (T)(2.0 * u6 + 4.0 * u12));
                 launches_++;
             }
@@ -1655,10 +987,7 @@ class Engine : public EngineBase {
                 if (vir && !vir_dev) memcpy(vir, host_sc + 1, 9 * sizeof(T));
             }
         }
-        MB_CUDA(cudaGetLastError());
-        if (path_ == 1) MB_TRY(check_overflow_sync());
-        else MB_CUDA(cudaStreamSynchronize(stream_));
-        return MB_OK;
+        return finish_call();
     }
 
     // ------------------------------------------------------------------------------------------
@@ -1674,24 +1003,23 @@ class Engine : public EngineBase {
     int enqueue_step(const StepCfg& c, int do_cm_now, bool clear_cm_after_k1, bool capture,
                      cudaGraphConditionalHandle handle, cudaGraph_t graph, cudaGraph_t* body_out, bool host_rebuild_hint,
                      bool defer_cm = false) {
-        const bool dec = decomposed() && path_ == 1;
-        const int s0 = dec ? own_s0_ : 0, n_own = dec ? own_n_ : (int)n_;
+        const bool dec = dc_.decomposed() && path_ == 1;
+        const int s0 = dec ? dc_.own_s0_ : 0, n_own = dec ? dc_.own_n_ : (int)n_;
         const int nb = std::max(1, (n_own + 255) / 256);
-        const int vvb = std::max(1, std::min((n_own + 2 * VV_THREADS - 1) / (2 * VV_THREADS), 8 * sm_count_));  // two atoms per thread
         Control* ctl = d_ctl_.as<Control>();
         CmState<T>* cm = d_cm_.as<CmState<T>>();
         // decomposed run over peer memory (peer.cuh): K1 mirrors the boundary slots into the neighbours while it drifts
-        const unsigned long long epoch = dec ? ++epoch_ : 0ull;
-        const bool p2p_halo = dec && p2p_active() && !host_rebuild_hint;  // rebuild steps all-gather the state instead
+        const unsigned long long epoch = dec ? ++dc_.epoch_ : 0ull;
+        const bool p2p_halo = dec && dc_.p2p_active() && !host_rebuild_hint;  // rebuild steps all-gather the state instead
         PeerPush<T> push;
         memset(&push, 0, sizeof(push));
-        if (p2p_halo) push = make_push(epoch, true);
-        if (cm_deferred_epoch_) {  // the previous step left v_cm in the momentum all-to-all (no peer_cm_kernel)
-            push.cm_comm = comm_of(rank_);
-            push.cm_nranks = nranks_;
-            push.cm_epoch = cm_deferred_epoch_;
+        if (p2p_halo) push = dc_.make_push(epoch, true);
+        if (dc_.cm_deferred_epoch_) {  // the previous step left v_cm in the momentum all-to-all (no peer_cm_kernel)
+            push.cm_comm = dc_.comm_of(dc_.rank_);
+            push.cm_nranks = dc_.nranks_;
+            push.cm_epoch = dc_.cm_deferred_epoch_;
             push.cm_inv_mass = c.inv_mass;
-            cm_deferred_epoch_ = 0;
+            dc_.cm_deferred_epoch_ = 0;
         }
         prof_.begin(Prof::VV);
         const Thermo<T> th = thermo_in_k1(c);
@@ -1728,44 +1056,46 @@ class Engine : public EngineBase {
             if (host_rebuild_hint) {
                 // neighbour rebuild on a decomposed box: replicate positions and velocities, rebuild (identical sort on every
                 // rank, lists only for the owned slab), then refresh the slot ranges and halo segments
-                MB_TRY(allgather_state());
+                MB_TRY(dc_.allgather_state(g_, d_pos4_.as<T4>(), d_vel4_.as<T4>()));
                 MB_TRY(set_flag_rebuild());
                 MB_TRY(enqueue_rebuild(true, false));
-                MB_TRY(update_ownership());
+                MB_TRY(dc_.update_ownership(g_, d_cell_start_.as<int>()));
             } else if (p2p_halo) {
-                gate_ = make_wait(epoch);  // the force kernel's CTAs wait for the neighbours' pushes of this epoch
+                dc_.gate_ = dc_.make_wait(epoch);  // the force kernel's CTAs wait for the neighbours' pushes of this epoch
             } else {
-                MB_TRY(halo_exchange());
+                MB_TRY(dc_.halo_exchange(d_pos4_.as<T4>()));
+                for (auto& sg : dc_.halo_recv_) MB_TRY(ext_fill(sg.start, sg.count));  // received slots -> extended array (+ ghost copies)
             }
         } else {
             if (rebuild_every_ == 0 || host_rebuild_hint) MB_TRY(enqueue_rebuild(true, false));
         }
-        const int s0b = dec ? own_s0_ : 0, n_ownb = dec ? own_n_ : (int)n_;  // ownership may have changed in the rebuild
+        const int s0b = dec ? dc_.own_s0_ : 0, n_ownb = dec ? dc_.own_n_ : (int)n_;  // ownership may have changed in the rebuild
         const int nb2 = std::max(1, (n_ownb + 255) / 256);
         const int vvb2 = std::max(1, std::min((n_ownb + 2 * VV_THREADS - 1) / (2 * VV_THREADS), 8 * sm_count_));
-        if (path_ == 0) MB_TRY(launch_allpairs(false, d_pos4_.as<T4>(), d_lj2_.as<T2>(), d_f4_.as<T4>()));
+        if (path_ == 0) MB_TRY(launch_allpairs(false));
         else MB_TRY(launch_force(false, dec));
         MB_TRY(launch_bonded(false));
-        const bool p2p_sig = dec && p2p_active();  // (after a rebuild: the new ownership's peers)
+        const bool p2p_sig = dec && dc_.p2p_active();  // (after a rebuild: the new ownership's peers)
         PeerSignal sig;
         memset(&sig, 0, sizeof(sig));
-        if (p2p_sig) sig = make_signal(epoch, do_cm_now != 0);
+        if (p2p_sig) sig = dc_.make_signal(epoch, do_cm_now != 0);
         prof_.begin(Prof::VV);
         vv_kick2_kernel<T><<<vvb2, VV_THREADS, 0, stream_>>>(s0b, n_ownb, c.dt_half, do_cm_now, c.inv_mass, d_f4_.as<T4>(), d_mass_.as<T>(),
                                                              d_vel4_.as<T4>(), d_partial_.as<double>(), ctl, cm, 0,
-                                                             dec ? d_mom_.as<double>() : nullptr, sig);
+                                                             dec ? dc_.mom() : nullptr, sig);
         prof_.end(Prof::VV);
         launches_++;
         if (p2p_sig && do_cm_now && defer_cm && !c.thermostat) {
-            cm_deferred_epoch_ = epoch;  // the next step's K1 adds the slabs' sums itself
+            dc_.cm_deferred_epoch_ = epoch;  // the next step's K1 adds the slabs' sums itself
         } else if (p2p_sig && do_cm_now) {
             // sum(m v) of all slabs arrived by peer stores: add them in rank order
-            peer_cm_kernel<T><<<1, 32, 0, stream_>>>(comm_of(rank_), nranks_, epoch, c.inv_mass, cm);
+            peer_cm_kernel<T><<<1, 32, 0, stream_>>>(dc_.comm_of(dc_.rank_), dc_.nranks_, epoch, c.inv_mass, cm);
             launches_++;
         } else if (dec && do_cm_now) {
             // global sum(m v): one 24-byte all-reduce per step, then v_cm for the lazy subtraction
-            MB_NCCL(g_nccl.AllReduce(d_mom_.as<double>(), d_mom_.as<double>() + 4, 3, ncclDouble, ncclSum, comm_, stream_));
-            cm_from_sum_kernel<T><<<1, 1, 0, stream_>>>(d_mom_.as<double>() + 4, c.inv_mass, cm);
+            double* mom = dc_.mom();
+            MB_NCCL(g_nccl.AllReduce(mom, mom + 4, 3, ncclDouble, ncclSum, dc_.comm_, stream_));
+            cm_from_sum_kernel<T><<<1, 1, 0, stream_>>>(mom + 4, c.inv_mass, cm);
             launches_++;
         }
         if (c.thermostat && !thermo_in_k1(c).on) {
@@ -1780,7 +1110,7 @@ class Engine : public EngineBase {
     Thermo<T> thermo_in_k1(const StepCfg& c) const {
         Thermo<T> th;
         memset(&th, 0, sizeof(th));
-        if (c.thermostat && !decomposed()) {
+        if (c.thermostat && !dc_.decomposed()) {
             th.on = 1;
             th.n = (int)n_;
             th.kT = c.kT;
@@ -1854,7 +1184,6 @@ class Engine : public EngineBase {
         MB_TRY(prepare());
         if (!coords || !vels || !p) return set_error(MB_ERR_INVALID, "null argument");
         if (p->n_steps < 0 || !(p->dt > 0)) return set_error(MB_ERR_INVALID, "n_steps < 0 or dt <= 0");
-        const bool c_dev = is_device_ptr(coords), v_dev = is_device_ptr(vels);
         const T* xc = nullptr;
         const T* vc = nullptr;
         MB_TRY(view_in(coords, 3 * (size_t)n_, d_stage_a_, &xc));
@@ -1874,10 +1203,7 @@ class Engine : public EngineBase {
         c.prob = p->andersen_prob;
         c.do_cm = (p->remove_cm_every == 0) ? 0 : (p->remove_cm_every == 1 ? 1 : -1);
         if (path_ == 0) {
-            init_slots_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, xc, d_charge_in_.as<T>(), d_ljp_in_.as<T2>(), d_mass_in_.as<T>(),
-                                                          d_pos4_.as<T4>(), d_vel4_.as<T4>(), d_lj2_.as<T2>(), d_orig_.as<int>(),
-                                                          d_inv_orig_.as<int>(), d_mass_.as<T>(), d_xref4_.as<T4>());
-            launches_++;
+            init_slots(xc);
             // velocities + wrap through ingest with an identity order (geometry only needs L)
             Geom<T> g0;
             memset(&g0, 0, sizeof(g0));
@@ -1894,13 +1220,13 @@ class Engine : public EngineBase {
         } else {
             MB_TRY(sync_state_from(xc, vc));
             c.skin_half2 = g_.skin_half2;  // geometry is chosen by the first build
-            c.flag_ptr = (rebuild_every_ == 0 && !decomposed()) ? &ctl->rebuild : &ctl->disp;
+            c.flag_ptr = (rebuild_every_ == 0 && !dc_.decomposed()) ? &ctl->rebuild : &ctl->disp;
         }
         // step bookkeeping lives on the device (tail of Control)
         {
             struct Tail { int rebuild_every; long long step, init_step; unsigned int rng[4]; unsigned int max_disp2_bits, call_max_disp2_bits; } t;
             static_assert(sizeof(Tail) == sizeof(Control) - offsetof(Control, rebuild_every), "Control tail layout");
-            t.rebuild_every = (decomposed() && path_ == 1) ? 0 : rebuild_every_;  // decomposed: the host counts the interval
+            t.rebuild_every = (dc_.decomposed() && path_ == 1) ? 0 : rebuild_every_;  // decomposed: the host counts the interval
             t.step = p->init_step;
             t.init_step = p->init_step;
             t.rng[0] = (unsigned int)p->rng_ctr1; t.rng[1] = (unsigned int)(p->rng_ctr1 >> 32);
@@ -1911,8 +1237,8 @@ class Engine : public EngineBase {
                                     cudaMemcpyHostToDevice, stream_));
             MB_CUDA(cudaStreamSynchronize(stream_));  // t is a local
         }
-        cm_deferred_epoch_ = 0;
-        adapt_span_ = since_rebuild_;
+        dc_.cm_deferred_epoch_ = 0;
+        dc_.adapt_span_ = dc_.since_rebuild_;
         bool cm_pending = false;  // host mirror of cm->valid
         if (p->init_step == 0 && p->remove_cm_every != 0) {
             // remove_CM_motion! before the first force evaluation (simulators.jl:563): zero-length kick
@@ -1922,29 +1248,29 @@ class Engine : public EngineBase {
             launches_++;
             cm_pending = true;
         }
-        const bool dec = decomposed() && path_ == 1;
-        if (dec && pme_on_) return set_error(MB_ERR_INVALID, "PME is not available in decomposed (multi-GPU) runs yet");
+        const bool dec = dc_.decomposed() && path_ == 1;
+        if (dec && pme_.on_) return set_error(MB_ERR_INVALID, "PME is not available in decomposed (multi-GPU) runs yet");
         if (dec) {
             // lists built from here on cover only the owned slab
-            build_b0_ = own_b0_;
-            build_nb_ = own_nb_;
-            MB_TRY(p2p_setup());  // collective; falls back to the NCCL transport on every rank if any mapping fails
+            dc_.build_b0_ = dc_.own_b0_;
+            dc_.build_nb_ = dc_.own_nb_;
+            MB_TRY(dc_.p2p_setup(d_pos4e_.p, env_.p2p));  // collective; falls back to the NCCL transport on every rank if any mapping fails
         }
-        if (path_ == 0) MB_TRY(launch_allpairs(false, d_pos4_.as<T4>(), d_lj2_.as<T2>(), d_f4_.as<T4>()));
+        if (path_ == 0) MB_TRY(launch_allpairs(false));
         else MB_TRY(launch_force(false, dec));
         MB_TRY(launch_bonded(false));
         if (dec) {
-            const unsigned long long e0 = ++epoch_;  // this force evaluation read the replicated state: tell the pushers
-            if (p2p_active()) {
-                peer_signal_kernel<<<1, 32, 0, stream_>>>(make_signal(e0, false));
+            const unsigned long long e0 = ++dc_.epoch_;  // this force evaluation read the replicated state: tell the pushers
+            if (dc_.p2p_active()) {
+                peer_signal_kernel<<<1, 32, 0, stream_>>>(dc_.make_signal(e0, false));
                 launches_++;
             }
         }
 
         // CUDA-graph path: static per-step sequence (remove_CM_motion in {0,1}, no stage timers requested)
-        bool use_graph = graph_enabled_ && !graph_failed_ && !prof_.enabled && c.do_cm >= 0 && p->n_steps >= 4 &&
+        bool use_graph = env_.graph && !graph_failed_ && !prof_.enabled && c.do_cm >= 0 && p->n_steps >= 4 &&
                          !(cm_pending && c.do_cm == 0) && !dec &&  // the decomposed step issues NCCL calls with per-rebuild sizes
-                         !pme_on_;                                  // cuFFT launches stay outside the captured step for now
+                         !pme_.on_;                                  // cuFFT launches stay outside the captured step for now
         if (use_graph) {
             GraphKey key{path_, c.do_cm, c.thermostat ? 1 : 0, geom_version_, rebuild_every_, p->dt, p->andersen_kT, p->andersen_prob, n_};
             if (!graph_exec_ || !(key == graph_key_)) {
@@ -1968,9 +1294,9 @@ class Engine : public EngineBase {
                 // decomposed: fixed interval counted on the host (identical on every rank), adapted per call from the displacements
                 bool hint;
                 if (dec) {
-                    hint = since_rebuild_ >= decomposed_interval();
-                    since_rebuild_ = hint ? 1 : since_rebuild_ + 1;
-                    adapt_span_ = std::max(adapt_span_, since_rebuild_);
+                    hint = dc_.since_rebuild_ >= dc_.interval(rebuild_every_);
+                    dc_.since_rebuild_ = hint ? 1 : dc_.since_rebuild_ + 1;
+                    dc_.adapt_span_ = std::max(dc_.adapt_span_, dc_.since_rebuild_);
                 } else {
                     hint = rebuild_every_ > 0 && k > 1 && (step_n - 1) % rebuild_every_ == 0;
                 }
@@ -1985,45 +1311,34 @@ class Engine : public EngineBase {
             launches_++;
         }
         if (dec) {
-            MB_TRY(allgather_state());  // every rank returns the whole system
-            build_nb_ = -1;
-            if (rebuild_every_ == 0) MB_TRY(adapt_interval());
+            MB_TRY(dc_.allgather_state(g_, d_pos4_.as<T4>(), d_vel4_.as<T4>()));  // every rank returns the whole system
+            dc_.build_nb_ = -1;
+            if (rebuild_every_ == 0) MB_TRY(dc_.adapt_interval(ctl, skin_, launches_));
         }
         // export
-        T* xo = c_dev ? reinterpret_cast<T*>(coords) : d_stage_a_.as<T>();
-        T* vo = v_dev ? reinterpret_cast<T*>(vels) : d_stage_c_.as<T>();
+        T *xo = nullptr, *vo = nullptr;
+        MB_TRY(view_out(coords, 3 * (size_t)n_, d_stage_a_, false, &xo));
+        MB_TRY(view_out(vels, 3 * (size_t)n_, d_stage_c_, false, &vo));
         export_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, path_ == 0 ? g_ap_ : g_, d_pos4_.as<T4>(), d_vel4_.as<T4>(), d_orig_.as<int>(), cm,
                                                   xo, vo);
         launches_++;
-        if (!c_dev) MB_CUDA(cudaMemcpyAsync(coords, xo, 3 * (size_t)n_ * sizeof(T), cudaMemcpyDeviceToHost, stream_));
-        if (!v_dev) MB_CUDA(cudaMemcpyAsync(vels, vo, 3 * (size_t)n_ * sizeof(T), cudaMemcpyDeviceToHost, stream_));
-        MB_CUDA(cudaGetLastError());
-        if (path_ == 1) MB_TRY(check_overflow_sync());
-        else MB_CUDA(cudaStreamSynchronize(stream_));
-        return MB_OK;
+        MB_TRY(view_out_done(coords, xo, 3 * (size_t)n_));
+        MB_TRY(view_out_done(vels, vo, 3 * (size_t)n_));
+        return finish_call();
     }
 
     // ------------------------------------------------------------------------------------------
     int remove_cm(void* vels) override {
         MB_TRY(prepare());
         if (!vels) return set_error(MB_ERR_INVALID, "null velocities");
-        const bool dev = is_device_ptr(vels);
-        const T* vc = nullptr;
-        MB_TRY(view_in(vels, 3 * (size_t)n_, d_stage_c_, &vc));
-        const int nb = (int)((n_ + 255) / 256);
-        MB_CUDA(d_partial_.ensure((size_t)nb * 3 * sizeof(double)));
-        momentum_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, vc, d_mass_in_.as<T>(), d_partial_.as<double>());
+        T* v = nullptr;
+        MB_TRY(view_out(vels, 3 * (size_t)n_, d_stage_c_, true, &v));
+        double s[3];
+        MB_TRY(reduce_to_host(momentum_kernel<T>, v, 3, s));
+        subtract_velocity_kernel<T><<<(int)((n_ + 255) / 256), 256, 0, stream_>>>((int)n_, (T)(s[0] / total_mass_), (T)(s[1] / total_mass_),
+                                                                                (T)(s[2] / total_mass_), v);
         launches_++;
-        std::vector<double> part((size_t)nb * 3);
-        MB_CUDA(cudaMemcpyAsync(part.data(), d_partial_.p, part.size() * sizeof(double), cudaMemcpyDeviceToHost, stream_));
-        MB_CUDA(cudaStreamSynchronize(stream_));
-        double s[3] = {0, 0, 0};
-        for (int b = 0; b < nb; b++) for (int d = 0; d < 3; d++) s[d] += part[3 * (size_t)b + d];
-        T* vw = const_cast<T*>(vc);
-        subtract_velocity_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, (T)(s[0] / total_mass_), (T)(s[1] / total_mass_),
-                                                             (T)(s[2] / total_mass_), vw);
-        launches_++;
-        if (!dev) MB_CUDA(cudaMemcpyAsync(vels, vw, 3 * (size_t)n_ * sizeof(T), cudaMemcpyDeviceToHost, stream_));
+        MB_TRY(view_out_done(vels, v, 3 * (size_t)n_));
         MB_CUDA(cudaStreamSynchronize(stream_));
         return MB_OK;
     }
@@ -2032,17 +1347,7 @@ class Engine : public EngineBase {
         if (!vels || !out) return set_error(MB_ERR_INVALID, "null argument");
         const T* vc = nullptr;
         MB_TRY(view_in(vels, 3 * (size_t)n_, d_stage_c_, &vc));
-        const int nb = (int)((n_ + 255) / 256);
-        MB_CUDA(d_partial_.ensure((size_t)nb * 3 * sizeof(double)));
-        kinetic_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, vc, d_mass_in_.as<T>(), d_partial_.as<double>());
-        launches_++;
-        std::vector<double> part(nb);
-        MB_CUDA(cudaMemcpyAsync(part.data(), d_partial_.p, part.size() * sizeof(double), cudaMemcpyDeviceToHost, stream_));
-        MB_CUDA(cudaStreamSynchronize(stream_));
-        double s = 0;
-        for (double v : part) s += v;
-        *out = s;
-        return MB_OK;
+        return reduce_to_host(kinetic_kernel<T>, vc, 1, out);
     }
     // kinetic energy tensor 1/2 sum m v (x) v (src/energy.jl:56-70) into out9 (3x3, symmetric, host doubles)
     int kinetic_tensor(const void* vels, double* out9) override {
@@ -2050,15 +1355,8 @@ class Engine : public EngineBase {
         if (!vels || !out9) return set_error(MB_ERR_INVALID, "null argument");
         const T* vc = nullptr;
         MB_TRY(view_in(vels, 3 * (size_t)n_, d_stage_c_, &vc));
-        const int nb = (int)((n_ + 255) / 256);
-        MB_CUDA(d_partial_.ensure((size_t)nb * 6 * sizeof(double)));
-        kinetic_tensor_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, vc, d_mass_in_.as<T>(), d_partial_.as<double>());
-        launches_++;
-        std::vector<double> part((size_t)nb * 6);
-        MB_CUDA(cudaMemcpyAsync(part.data(), d_partial_.p, part.size() * sizeof(double), cudaMemcpyDeviceToHost, stream_));
-        MB_CUDA(cudaStreamSynchronize(stream_));
-        double k[6] = {0, 0, 0, 0, 0, 0};
-        for (int b = 0; b < nb; b++) for (int d = 0; d < 6; d++) k[d] += part[6 * (size_t)b + d];
+        double k[6];
+        MB_TRY(reduce_to_host(kinetic_tensor_kernel<T>, vc, 6, k));
         out9[0] = k[0]; out9[4] = k[1]; out9[8] = k[2];
         out9[1] = out9[3] = k[3]; out9[2] = out9[6] = k[4]; out9[5] = out9[7] = k[5];
         return MB_OK;
@@ -2067,17 +1365,13 @@ class Engine : public EngineBase {
     int random_velocities(void* vels, double kT, uint64_t ctr1, uint64_t key) override {
         MB_TRY(prepare());
         if (!vels || !(kT >= 0)) return set_error(MB_ERR_INVALID, "mb_random_velocities: null velocities or negative kT");
-        const bool dev = is_device_ptr(vels);
-        T* vo = reinterpret_cast<T*>(vels);
-        if (!dev) {
-            MB_CUDA(d_stage_c_.ensure(3 * (size_t)n_ * sizeof(T)));
-            vo = d_stage_c_.as<T>();
-        }
+        T* vo = nullptr;
+        MB_TRY(view_out(vels, 3 * (size_t)n_, d_stage_c_, false, &vo));
         const int nb = (int)((n_ + 255) / 256);
         random_velocities_kernel<T><<<nb, 256, 0, stream_>>>((int)n_, (T)kT, d_mass_in_.as<T>(), (uint32_t)ctr1, (uint32_t)(ctr1 >> 32),
                                                              (uint32_t)key, (uint32_t)(key >> 32), vo);
         launches_++;
-        if (!dev) MB_CUDA(cudaMemcpyAsync(vels, vo, 3 * (size_t)n_ * sizeof(T), cudaMemcpyDeviceToHost, stream_));
+        MB_TRY(view_out_done(vels, vo, 3 * (size_t)n_));
         MB_CUDA(cudaStreamSynchronize(stream_));
         return MB_OK;
     }
@@ -2100,8 +1394,8 @@ class Engine : public EngineBase {
         o->r_list = r_list_;
         o->kernel_launches = launches_;
         o->graph_mode = graph_used_ ? 1 : (graph_failed_ ? -1 : 0);
-        o->reserved_ = decomposed() ? auto_every_ : 0;
-        o->peer_transport = (decomposed() && p2p_active()) ? 1 : 0;
+        o->reserved_ = dc_.decomposed() ? dc_.auto_every_ : 0;
+        o->peer_transport = (dc_.decomposed() && dc_.p2p_active()) ? 1 : 0;
         prof_.collect();
         o->force_ms = prof_.ms[Prof::FORCE]; o->force_launches = prof_.count[Prof::FORCE];
         o->vv_ms = prof_.ms[Prof::VV]; o->vv_launches = prof_.count[Prof::VV];
@@ -2127,14 +1421,12 @@ class Engine : public EngineBase {
     }
 
    private:
-    int device_;
     cudaStream_t stream_;
     int sm_count_ = 148;
     size_t smem_optin_ = 232448;
+    const EnvSwitches env_;  // read at construction
     int64_t n_ = 0;
     std::vector<T> h_mass_, h_charge_, h_sigma_, h_eps_, h_eps_raw_;
-    double disp_rc_ = 0, disp_f6_ = 0, disp_f12_ = 0;  // LJDispersionCorrection (0 = off)
-    bool disp_ready_ = false;
     double box_[3];
     std::vector<mb_inter_t> inters_;
     std::vector<int> ex_ptr_, ex_idx_, sp_ptr_, sp_idx_;
@@ -2142,53 +1434,23 @@ class Engine : public EngineBase {
     double r_list_ = 0, skin_ = 0, cap_scale_ = 1.0, total_mass_ = 0;
     int rebuild_every_ = 0;
     int user_b_[3] = {0, 0, 0};
-    int lpa_ = 8;
-    bool dirty_ = true, have_list_ = false, slots_init_ = false;
+    bool dirty_ = true, have_list_ = false;
     int cutm_ = CUTM_PLAIN;  // cutoff family of the kernel variant (pair.cuh)
     int path_ = 0;
     PairParams<T> P_;
     Geom<T> g_, g_ap_;
     Tric<T> tric_ = {};  // TriclinicBoundary (on = 0: cubic / rectangular box)
-    Control last_ctl_;
     int64_t launches_ = 0, n_force_evals_ = 0, n_steps_ = 0, graph_step_launches_ = 0;
     Prof prof_;
     cudaGraph_t graph_ = nullptr;
     cudaGraphExec_t graph_exec_ = nullptr;
     GraphKey graph_key_;
-    bool graph_enabled_ = true, graph_failed_ = false, graph_used_ = false, own_stream_ = false;
+    bool graph_failed_ = false, graph_used_ = false, own_stream_ = false;
     int geom_version_ = 0;
-    // spatial decomposition (z-slabs of cell layers; one rank per GPU)
-    ncclComm_t comm_ = nullptr;
-    int rank_ = 0, nranks_ = 1;
-    int own_b0_ = 0, own_nb_ = 0;        // this rank's bricks (static for a geometry)
-    bool own_valid_ = false;             // ownership derived from the current sort
-    int since_rebuild_ = 0;              // MD steps since the last rebuild of a decomposed run (host count, same on every rank)
-    int adapt_span_ = 0;                 // longest such count within the current call
-    int build_b0_ = 0, build_nb_ = -1;   // brick range the list builder covers (-1 = all)
-    int own_s0_ = 0, own_n_ = 0;         // this rank's slots (changes at every rebuild)
-    int auto_every_ = 20;                // rebuild interval of decomposed runs when the policy is displacement-triggered
-    std::vector<int> layer_start_;       // slot index of the first atom of every cell layer (ncz + 1)
-    std::vector<DecompSeg> halo_send_, halo_recv_;
-    DevBuf d_layer_start_, d_mom_;
-    // peer-memory transport (peer.cuh): IPC-mapped position arrays and PeerComm blocks of the other ranks
-    bool p2p_ = false;
-    void* p2p_pos_base_ = nullptr;            // the d_pos4_ allocation the peers have mapped
-    DevBuf d_comm_, d_ipc_;
-    std::vector<void*> peer_pos_, peer_comm_; // [rank]; own entries point at the local buffers
-    unsigned long long epoch_ = 0;            // force evaluations of decomposed runs (same on every rank)
-    bool plan_fits_ = false;
-    PeerWait gate_ = {};
-    unsigned long long cm_deferred_epoch_ = 0;
-    int plan_key_[3] = {-1, -1, -1};
-    int64_t sp_n_[3] = {0, 0, 0};
-    DevBuf d_sp_idx_k_[3], d_sp_par_k_[3], d_sp_partial_, d_sp_energy_;
-    // PME (pme.cuh)
-    bool pme_on_ = false, pme_ready_ = false;
-    double pme_rc_ = 0, pme_tol_ = 0, pme_epsr_ = 1, pme_alpha_ = 0, pme_self_e_ = 0, pme_ke_ = 138.93545764;
-    PmeGeom pme_g_ = {{0, 0, 0}, {0, 0, 0}};
-    int pme_plan_ = -1;
-    std::vector<int> pme_pairs_;
-    DevBuf d_pme_grid_, d_pme_bsm_[3], d_pme_partial_, d_pme_pairs_;
+    Decomp<T> dc_;         // multi-GPU state and transport (decomp.cuh)
+    BondedHost<T> bonded_; // specific interaction lists (specific.cuh)
+    PmeHost<T> pme_;       // PME (pme_host.cuh)
+    Dispersion disp_;      // LJDispersionCorrection (specific.cuh)
     DevBuf d_mass_in_, d_charge_in_, d_ljp_in_;
     DevBuf d_pos4_, d_vel4_, d_f4_, d_xref4_, d_lj2_, d_orig_, d_inv_orig_, d_mass_;
     DevBuf d_pos4_t_, d_vel4_t_, d_lj2_t_, d_orig_t_, d_mass_t_;
@@ -2200,8 +1462,6 @@ class Engine : public EngineBase {
     DevBuf d_ext_of_, d_gptr_, d_ghosts_, d_pos4e_, d_lj2e_, d_orig_e_;    // slot -> extended map, ghost table, extended arrays
     DevBuf d_task_tab_, d_sched_;  // per-brick task tables; brick ticket + finished-CTA counter of the force kernel
     int force_grid_ = 0;           // CTAs of the last force launch (= number of energy partials)
-    bool static_sched_ = false;    // MOLLYB200_STATIC_SCHED=1: round-robin bricks instead of tickets
-    double max_rc_ = 0;
     DevBuf d_partial_, d_pe_partial_;
 };
 

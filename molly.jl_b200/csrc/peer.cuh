@@ -90,11 +90,6 @@ struct PeerWait {
     unsigned long long epoch;
 };
 
-// gate in front of the force kernel: one lane per peer that pushes into this rank
-__global__ void peer_wait_kernel(PeerWait w) {
-    if ((int)threadIdx.x < w.n) spin_until(w.flag[threadIdx.x], w.epoch);
-}
-
 // stand-alone signal (after the force evaluation that precedes the first step of a call)
 __global__ void peer_signal_kernel(PeerSignal s) {
     if ((int)threadIdx.x < s.n_peer) {
